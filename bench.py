@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- WSPR windows/s through coarse search + fine sync + soft-symbol demodulation.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--windows M]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--windows M] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[2], the largest single-GPU configuration): M = 10 000
 independent synthetic WSPR windows per GPU (45 000 complex64 samples at 375 sps each, 3.6 GB,
@@ -43,6 +43,13 @@ the reference arm, the cpu_baseline leg and the verify leg only, never inside a 
 --impl reference times the reference's own CPU implementation (oracle/_ref, the unmodified
 sources; the C restatement if it was not built) on all host cores, on a bounded sample that is a
 prefix of the GPU arm's batch.
+
+--steps K sets the number of timed steps of every arm.  --dump-outputs DIR writes the headline step's
+results for rank 0's batch (dump_outputs) as DIR/<name>.npy, so that two builds can be compared output
+for output: the inputs are seeded and the same on every run with the same arguments.  The timed steps
+leave their results on the device, where the library offers no way to read them back, so after the
+timed steps the same call runs once more on the same device samples with its results fetched; that
+call is untimed, and its candidate count must equal the last timed step's.
 """
 import argparse
 import json
@@ -196,6 +203,46 @@ def measured_peaks():
 
 def whales_fixture():
     return np.load(os.path.join(ROOT, "tests", "golden", "whales_375sps.npy"))
+
+
+DUMP_BYTES = 64 << 20
+DUMP_WINDOWS, DUMP_CANDIDATES, DUMP_SOFT_CANDIDATES = 1 << 18, 1 << 15, 1 << 11
+
+
+def _sample(n, k, seed):
+    """all of range(n), or a fixed seeded sample of k of them in increasing order"""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def dump_outputs(path, npk, cands, refined, jig, soft):
+    """writes the arrays coarse_fine returns (npk, cands, refined, jig, soft) as path/<name>.npy, one file per
+    field, in float32 (float fields, soft symbols) or float64 (integer fields, indices).  Where there are more
+    windows or candidates than DUMP_BYTES holds, a fixed seeded sample of them is written; *_index.npy says which.
+    Union fields are written where they are defined (lin_drift for linear candidates, V1, V2, p1, p2 for
+    nonlinear ones) and are 0 elsewhere; candidate_t.drift is never written by the reference and is left out."""
+    wi = _sample(len(npk), DUMP_WINDOWS, 1)
+    ci = _sample(len(cands), DUMP_CANDIDATES, 2)
+    si = _sample(len(cands), DUMP_SOFT_CANDIDATES, 3)
+    c, r, j = cands[ci], refined[ci], jig[ci]
+    lin, nonlin = c["m_type"] == 0, c["m_type"] == 1
+    f32, f64 = (lambda a: np.asarray(a, np.float32)), (lambda a: np.asarray(a, np.float64))
+    out = dict(counts=f64([len(npk), len(cands)]), window_index=f64(wi), npk=f64(npk[wi]), cand_index=f64(ci),
+               cand_freq=f32(c["freq"]), cand_snr=f32(c["snr"]), cand_sync=f32(c["sync"]), cand_shift=f64(c["shift"]),
+               cand_m_type=f64(c["m_type"]), cand_lin_drift=f32(np.where(lin, c["lin_drift"], 0)),
+               cand_V1=f64(np.where(nonlin, c["V1"], 0)), cand_V2=f64(np.where(nonlin, c["V2"], 0)),
+               cand_p1=f64(np.where(nonlin, c["p1"], 0)), cand_p2=f64(np.where(nonlin, c["p2"], 0)),
+               refined_f1=f32(r["f1"]), refined_shift1=f64(r["shift1"]), refined_drift1=f32(r["drift1"]),
+               refined_sync1=f32(r["sync1"]), refined_worth_a_try=f64(r["worth_a_try"]),
+               jig_sync=f32(j["sync"]), jig_rms=f32(j["rms"]), jig_shift=f64(j["shift"]), jig_gate=f64(j["gate"]),
+               soft_index=f64(si), soft=f32(soft[si]))
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_BYTES, total
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    return total
 
 
 # ------------------------------------------------------------------ reference arm
@@ -365,6 +412,12 @@ def run_ours(args):
     launches = ctx.launch_count() - l0
     st = stage_ms / steps
     ncand_dev = totals[-1]
+    if args.dump_outputs and rank == 0:
+        # a recompute: the timed calls leave their results on the device, and the library has no call to read them
+        # back; the same call on the same device samples, untimed and with results fetched, returns them
+        res = ctx.coarse_fine(dptr, nwin=nwin, stride=FL, out=out_bufs)
+        assert len(res[1]) == ncand_dev, (len(res[1]), ncand_dev)
+        dump_outputs(args.dump_outputs, *res)
     for _ in range(min(warmup, 1) or 1):
         step_e2e()
     e2e_counts = [nwin] * world
@@ -583,13 +636,13 @@ def bench_receiver(H, ub, ctx, xs_host, nwin, out_bufs, truth, dec_full, steps):
 
     one()
     H.barrier()
-    t = [one() for _ in range(max(1, min(steps, 2)))]
+    t = [one() for _ in range(steps)]
     sec = float(np.mean(t))
     tt = torch.tensor([sec], device=H.dev)
     if H.world > 1:
         H.dist.all_reduce(tt, op=H.dist.ReduceOp.MAX)
     full = {g: bytes(m) for g, m, _ in dec_full}
-    return dict(value=H.world * nwin / float(tt.item()), unit="windows/s", host_threads=cores,
+    return dict(value=H.world * nwin / float(tt.item()), unit="windows/s", steps=steps, host_threads=cores,
                 seconds=dict(device_first_jiggle=stats["device_1"], host_decode_first=stats["decode_1"],
                              device_other_jiggles=stats["device_2"], host_decode_rest=stats["decode_2"]),
                 candidates=stats["cands"], retried=stats["retry"], messages=len(stats["msgs"]),
@@ -602,7 +655,7 @@ def bench_stream(H, ub, synth, rates, verify_jobs, name, W, stride, nverify):
     """one synthetic stream (a frame every 45 000 samples), W windows every `stride` samples, contiguous slices per rank"""
     from uwspr_b200.sharding import balanced_counts, gather_floats, shard_range
     args, world, rank, dev = H.args, H.world, H.rank, H.dev
-    steps = max(1, min(args.steps, 3)) if W >= 50000 and world == 1 else args.steps
+    steps = args.steps
     # device-resident arm: equal contiguous slices
     lo, hi = shard_range(W, rank, world)
     # host-fed arm: contiguous slices in proportion to the host-link rates measured by the headline arm
@@ -786,7 +839,13 @@ def main():
     ap.add_argument("--skip", default="", help="comma list of sub-records to leave out: overlap50,sliding9,array64,receiver")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-balance", action="store_true", help="host-fed arms at N > 1: equal split instead of link-rate balanced")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, recompute the headline step once with results fetched and write them "
+                                                           "(rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's results; the reference arm has none")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -14,7 +14,7 @@ if PKG not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run with -m gpu on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs oracle/_ref built from /root/reference")
+    config.addinivalue_line("markers", "reference: compares with the reference (live where oracle/_ref is built, else recorded)")
 
 
 @pytest.fixture(scope="session")

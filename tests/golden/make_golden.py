@@ -16,6 +16,13 @@ Outputs (committed; the GPU box has no /root/reference):
                    deinterleaver and the decoder.
 Cases = the four fixture windows (FDR hbw=10, maxdrift=0, thr=10, as in
 examples/WaveFilePlusNoiseDecode.grc) + seeded synthetic windows at maxdrift 0 and 4.
+
+    python tests/golden/make_golden.py --reference-cases [--from-repository]
+
+writes only recorded_cases.npz: the reference's side of every case in tests/golden/reference_cases.py (what the
+comparisons with the reference compare against where oracle/_ref is not built).  It needs oracle/_ref; with
+--from-repository the answers come from this repository's side of the same cases instead, and the file's
+`source` entry says so.
 """
 import os
 import sys
@@ -24,6 +31,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "gr-uwspr_b200"))
 from oracle import ref_binding as rb  # noqa: E402
 from oracle import testdata as td  # noqa: E402
 
@@ -59,7 +67,25 @@ def write_whales():
     print("whales_375sps", y.shape, float(np.sqrt((np.abs(y) ** 2).mean())))
 
 
+def write_reference_cases(ref):
+    from tests.golden import reference_cases as rc
+    if ref and not rb.available():
+        raise SystemExit("oracle/_ref is not built (make -C oracle ref); --from-repository records this repository's side")
+    golden = np.load(os.path.join(OUT, "golden.npz"))
+    windows = {n: np.load(os.path.join(OUT, "win_%s.npy" % n)) for n in ("ve3emb_c2", "mix_whales")}
+    out = dict(source=np.array("oracle/_ref (the unmodified upstream sources)" if ref else
+                               "this repository: the oracle's C restatement; the library's unpacker and message-log formatter"))
+    for name in rc.CASES:
+        for k, v in rc.compute(name, ref, golden, windows).items():
+            out[name + "/" + k] = v
+    np.savez_compressed(rc.RECORDED, **out)
+    print("wrote", rc.RECORDED, os.path.getsize(rc.RECORDED), "bytes, source:", out["source"])
+
+
 def main():
+    if "--reference-cases" in sys.argv:
+        write_reference_cases(ref="--from-repository" not in sys.argv)
+        return
     write_whales()
     if "--whales-only" in sys.argv:
         return

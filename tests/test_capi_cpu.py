@@ -11,6 +11,7 @@ import pytest
 import uwspr_b200 as ub
 from oracle import port_binding as ob
 from oracle import testdata as td
+from tests.golden import reference_cases as rc
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -95,27 +96,13 @@ def test_shard_ranges():
     assert stream_span(2, 5, 22500, 45000) == (45000, 4 * 22500 + 45000)
 
 
-def test_message_log_text_matches_reference_file(lib, golden, golden_windows, tmp_path):
+def test_message_log_text_matches_reference_file(lib, golden, golden_windows):
     """the reference block appends to ./messagelog.txt on every decode (sync_and_demodulate_impl.cc:507-526);
-    the same candidates and blobs through uwspr_b200_format_message_log give the same lines"""
-    from oracle import ref_binding as rb
-    from uwspr_b200.binding import format_message_log
-    if not rb.available():
-        pytest.skip("oracle/_ref not built")
-    sd = rb.RefSD(logdir=str(tmp_path))
-    want = ""
-    frame = 0
-    for name in ("ve3emb_c2", "mix_whales"):   # a nonlinear and a linear candidate
-        cands = golden[name + "/cands"].view(rb.CAND_DTYPE).reshape(-1)
-        blobs, calls, fanos = sd.demodulate(golden_windows[name], cands)
-        assert len(blobs) == 1
-        frame += 1
-        decoded = cands[0]                     # in both fixtures the first candidate is the one that decodes
-        want += format_message_log(frame, decoded, blobs[0])
-    text = open(tmp_path / "messagelog.txt").read()
-    got = "".join(l + "\n" for l in text.split("\n")[2:] if not l.startswith(("Handoff time", "Elapsed time")))
-    # got now starts after the "Start time" line and its blank line; strip the trailing split artefact
-    assert got.rstrip("\n") + "\n\n" == want
+    the same candidates and blobs through uwspr_b200_format_message_log give the same lines (the reference's
+    file live where oracle/_ref is built, else as recorded)"""
+    want = rc.reference("message_log", golden, golden_windows)
+    rc.assert_same(rc.compute("message_log", False, golden, golden_windows), want)
+    assert bytes(want["text"]).decode("latin1").count("Frame: ") == 2
 
 
 def test_unpacker_known_answers(lib):
@@ -127,25 +114,12 @@ def test_unpacker_known_answers(lib):
 
 def test_unpacker_against_reference_all_message_types(lib):
     """random 50-bit payloads cover type 1, type 2 (prefix/suffix) and type 3 (hashed call) paths, with the
-    callsign hash table evolving identically on both sides (lib/helpers.cc:494-590)"""
-    from oracle import ref_binding as rb
-    if not rb.available():
-        pytest.skip("oracle/_ref not built")
-    mine, ref = ub.WSPR_unpacker(), rb.RefUnpacker()
-    rng = np.random.default_rng(50)
-    kinds = set()
-    for trial in range(20000):
-        m = rng.integers(0, 256, 7).astype(np.uint8)
-        m[6] &= 0xC0
-        if trial % 3 == 0:                     # bias towards valid callsigns / type 1
-            m[:4] = np.frombuffer(bytes.fromhex("d42c73eb"), np.uint8)
-            m[3] = (m[3] & 0xF0) | int(rng.integers(0, 16))
-        a, b = mine.unpack(m), ref.unpack(m)
-        assert a == b, (m.tobytes().hex(), a, b)
-        if b[1]:
-            kinds.add("3" if b[1].startswith("<") else "2" if "/" in b[1] else "1")
+    callsign hash table evolving identically on both sides (lib/helpers.cc:494-590); the reference answers live
+    where oracle/_ref is built, else as recorded"""
+    want = rc.reference("unpacker")
+    rc.assert_same(rc.compute("unpacker", False), want)
+    kinds = {"3" if t.startswith("<") else "2" if "/" in t else "1" for t in rc.texts(want) if t}
     assert kinds == {"1", "2", "3"}
-    assert np.array_equal(mine.hashtab, ref.hashtab)
 
 
 def test_decode_batch_equals_candidate_loop_for_any_thread_count(lib):
@@ -209,11 +183,8 @@ def test_packer_and_channel_symbols_round_trip(lib, golden):
     rng = np.random.default_rng(3)
     letters = "ABCDEFGHIJKLMNOPQRSTUVWXYZ"
     u = ub.WSPR_unpacker()
-    try:
-        from oracle import ref_binding as rb
-        ru = rb.RefUnpacker() if os.path.exists("/root/reference") else None
-    except Exception:
-        ru = None
+    from oracle import ref_binding as rb
+    ru = rb.RefUnpacker() if rb.available() else None
     for trial in range(300):
         n_suffix = int(rng.integers(1, 4))
         if trial % 2:   # digit second: "K1ABC"
@@ -251,9 +222,6 @@ def test_c2_reader(lib, golden_windows, tmp_path):
         ub.read_c2(str(tmp_path / "short.c2"))
     with pytest.raises(ub.UwsprError):
         ub.read_c2(str(tmp_path / "missing.c2"))
-    ref = "/root/reference/examples/VE3EMB.c2"
-    if os.path.exists(ref):
-        assert ub.read_c2(ref)[0].tobytes() == x.tobytes()
 
 
 def test_frontend_and_batch_decoder_argument_checks(lib):
