@@ -1,6 +1,7 @@
 // C ABI of libuwspr_b200.so (include/uwspr_b200.h): context, constant tables, chunked
 // submission with copy/compute overlap.  No CPU fallback exists for the ported stages:
 // without a usable CUDA device uwspr_b200_create fails.
+#include <limits.h>
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -104,6 +105,17 @@ struct Buffers {
     float2 *twiddle = nullptr;
     uint32_t *off4 = nullptr;
     short *hyp_unique = nullptr;
+    // device decoder (uwspr_b200_decode_device), allocated by its first call for max_candidates
+    int *dec_first_ok = nullptr;            // [cap]: smallest jiggle that decoded so far
+    int *dec_tasks = nullptr;               // [cap * NJIG]: gated (candidate, jiggle) pairs
+    uint32_t *dec_task_cycles = nullptr;    // [cap * NJIG]
+    unsigned long long *dec_task_msg = nullptr;  // [cap * NJIG]: bytes 0..6 of a successful task's data
+    int *dec_counters = nullptr;            // task count, task cursor
+    uint8_t *dec_out = nullptr;             // decoded[cap], msg7[cap * 7], idt_used[cap], fano_cycles[cap]
+    short *mettab = nullptr;                // WSPR_METTAB
+    // raw decoder rows (uwspr_b200_fano_batch): symbols and outputs, grown on demand
+    uint8_t *rows = nullptr;
+    size_t rows_cap = 0;
 };
 
 }  // namespace
@@ -133,6 +145,9 @@ struct uwspr_b200_ctx {
     std::string err;
     bool debug_ps = false;
     bool have_coarse = false;  // device candidate list valid for a following fine call
+    bool have_fine = false;    // b.refined / b.jig / b.soft hold last_total candidates x last_jig_count jiggles
+    int last_jig_count = 0;
+    int fano_grid = 0;         // resident blocks of the decoder kernel
     int last_nwin = 0, last_total = 0;
     const float *last_samples = nullptr;
     int64_t last_stride = 0;
@@ -315,6 +330,8 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
         if (total_out) *total_out = 0;
         ctx->last_total = 0;
         ctx->last_nwin = 0;
+        ctx->have_fine = do_fine;
+        ctx->last_jig_count = jig_count;
         return UWSPR_B200_OK;
     }
     // Device-resident input: one stream, chunks as large as the buffers allow (no tails between
@@ -568,6 +585,10 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
                         "kernels end %.3f ms, results on host %.3f ms\n", nwin, nchunks, c0, c1, k, ctx->ms[3]);
     }
     ctx->have_coarse = true;
+    // the fine path writes b.refined[g], b.jig[g * jig_count + t] and b.soft[(g * jig_count + t) * 162] at the
+    // call-wide candidate index g (the work list's running total), for host-fed and resident input alike
+    ctx->have_fine = do_fine;
+    ctx->last_jig_count = jig_count;
     ctx->last_nwin = nwin;
     ctx->last_total = total;
     ctx->last_samples = samples;
@@ -591,6 +612,7 @@ int run(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_stride
             if (q) cudaStreamSynchronize(q);
         cudaGetLastError();
         ctx->have_coarse = false;
+        ctx->have_fine = false;
         ctx->last_nwin = 0;
     }
     return rc;
@@ -726,9 +748,10 @@ int uwspr_b200_create(const uwspr_b200_params_t *params, uwspr_b200_ctx **ctx_ou
     CUC(cudaEventCreate(&ctx->ev_cp1));
     CUC(cudaEventCreate(&ctx->ev_kend));
     CUC(cudaEventCreate(&ctx->ev_end));
-    if (uw_coarse_setup(d) || uw_fine_setup())
+    if (uw_coarse_setup(d) || uw_fine_setup() || uw_fano_setup())
         return bail(fail(ctx, UWSPR_B200_E_CUDA, "cannot reserve shared memory for the kernels (not an sm_100a device?)"));
     ctx->grid_coarse = ctx->sm_count * uw_coarse_blocks_per_sm(d);
+    ctx->fano_grid = ctx->sm_count * uw_fano_blocks_per_sm();
     {
         int bp = 1, bl = 1;
         uw_fine_blocks_per_sm(&bp, &bl);
@@ -756,7 +779,8 @@ void uwspr_b200_destroy(uwspr_b200_ctx *ctx)
     Buffers &b = ctx->b;
     void *ptrs[] = { b.x_stage[0], b.x_stage[1], b.x_stage[2], b.amp, b.ps_dbg, b.psavg, b.peaks, b.npk, b.base, b.items,
                      b.cands, b.refined, b.jig, b.soft, b.counters, b.fine_tickets, b.fine_state[0], b.fine_state[1], b.fine_state[2], b.fine_pbuf[0], b.fine_pbuf[1],
-                     b.fine_pbuf[2], b.fine_pe[0], b.fine_pe[1], b.fine_pe[2], b.fine_pbest[0], b.fine_pbest[1], b.fine_pbest[2], b.fine_tables[0], b.fine_tables[1], b.fine_tables[2], b.window, b.twiddle, b.off4, b.hyp_unique };
+                     b.fine_pbuf[2], b.fine_pe[0], b.fine_pe[1], b.fine_pe[2], b.fine_pbest[0], b.fine_pbest[1], b.fine_pbest[2], b.fine_tables[0], b.fine_tables[1], b.fine_tables[2], b.window, b.twiddle, b.off4, b.hyp_unique,
+                     b.dec_first_ok, b.dec_tasks, b.dec_task_cycles, b.dec_task_msg, b.dec_counters, b.dec_out, b.mettab, b.rows };
     for (void *q : ptrs)
         if (q) cudaFree(q);
     for (cudaEvent_t e : ctx->ev) cudaEventDestroy(e);
@@ -865,6 +889,177 @@ int uwspr_b200_wait(uwspr_b200_ctx *ctx)
     if (!ctx) return UWSPR_B200_E_PARAM;
     if (!ctx->pending.valid()) return fail(ctx, UWSPR_B200_E_STATE, "nothing was submitted");
     return ctx->pending.get();
+}
+
+}  // extern "C"
+
+namespace {
+
+int ensure_mettab(uwspr_b200_ctx *ctx)
+{
+    Buffers &b = ctx->b;
+    if (b.mettab) return UWSPR_B200_OK;
+    CU(cudaMalloc(&b.mettab, sizeof(WSPR_METTAB)));
+    // on the context's stream: the kernels run there, and that stream does not wait for the legacy default stream
+    CU(cudaMemcpyAsync(b.mettab, WSPR_METTAB, sizeof(WSPR_METTAB), cudaMemcpyHostToDevice, ctx->compute));
+    CU(cudaStreamSynchronize(ctx->compute));
+    return UWSPR_B200_OK;
+}
+
+int ensure_decoder(uwspr_b200_ctx *ctx)
+{
+    Buffers &b = ctx->b;
+    const int rc = ensure_mettab(ctx);
+    if (rc || b.dec_out) return rc;
+    const size_t cap = (size_t)ctx->max_candidates, ntask = cap * UWSPR_B200_NJIG;
+    CU(cudaMalloc(&b.dec_first_ok, cap * sizeof(int)));
+    CU(cudaMalloc(&b.dec_tasks, ntask * sizeof(int)));
+    CU(cudaMalloc(&b.dec_task_cycles, ntask * sizeof(uint32_t)));
+    CU(cudaMalloc(&b.dec_task_msg, ntask * sizeof(unsigned long long)));
+    CU(cudaMalloc(&b.dec_counters, 2 * sizeof(int)));
+    CU(cudaMalloc(&b.dec_out, cap * (1 + 7 + sizeof(int32_t) + sizeof(uint32_t))));
+    return UWSPR_B200_OK;
+}
+
+// (maxcycles * nbits + 1) * delta must fit in int32: the device decoder keeps its threshold in 32 bits (fano.cu)
+bool fano_domain(uint32_t nbits, int delta, uint32_t maxcycles)
+{
+    if (nbits < 32 || nbits > 81 || delta <= 0 || maxcycles < 1) return false;
+    const unsigned long long steps = (unsigned long long)maxcycles * nbits + 1;
+    return steps * (unsigned long long)delta <= (unsigned long long)INT32_MAX;
+}
+
+int decode_impl(uwspr_b200_ctx *ctx, const uwspr_b200_refined_t *refined, const uwspr_b200_jiggle_t *jig,
+                const uint8_t *soft, int space, int ncand, int jig_count, uint8_t *decoded, int8_t *messages7,
+                int32_t *idt_used, uint32_t *fano_cycles, int *ndecoded)
+{
+    CU(cudaSetDevice(ctx->device));
+    int rc = ensure_decoder(ctx);
+    if (rc) return rc;
+    Buffers &b = ctx->b;
+    cudaStream_t cs = ctx->compute;
+    if (refined) {
+        // the caller's inputs replace the fine results of the last call on the device
+        ctx->have_fine = false;
+        const cudaMemcpyKind k = space == UWSPR_B200_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+        const size_t n = (size_t)ncand;
+        CU(cudaMemcpyAsync(b.refined, refined, n * sizeof(uwspr_b200_refined_t), k, cs));
+        CU(cudaMemcpyAsync(b.jig, jig, n * jig_count * sizeof(uwspr_b200_jiggle_t), k, cs));
+        CU(cudaMemcpyAsync(b.soft, soft, n * jig_count * UW_NSYM, k, cs));
+    }
+    const size_t cap = (size_t)ctx->max_candidates;
+    uint8_t *d_dec = b.dec_out;
+    int8_t *d_msg = reinterpret_cast<int8_t *>(b.dec_out + cap);
+    int32_t *d_idt = reinterpret_cast<int32_t *>(b.dec_out + 8 * cap);
+    uint32_t *d_cyc = reinterpret_cast<uint32_t *>(b.dec_out + 12 * cap);
+    uw_launch_fano_candidates(b.refined, b.jig, b.soft, ncand, jig_count, b.mettab, b.dec_first_ok, b.dec_tasks,
+                              b.dec_counters, b.dec_task_cycles, b.dec_task_msg, ctx->fano_grid, d_dec, d_msg, d_idt, d_cyc, cs);
+    ctx->launches += jig_count > 0 ? 3 : 2;
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(decoded, d_dec, (size_t)ncand, cudaMemcpyDeviceToHost, cs));
+    CU(cudaMemcpyAsync(messages7, d_msg, (size_t)ncand * 7, cudaMemcpyDeviceToHost, cs));
+    if (idt_used) CU(cudaMemcpyAsync(idt_used, d_idt, (size_t)ncand * sizeof(int32_t), cudaMemcpyDeviceToHost, cs));
+    if (fano_cycles) CU(cudaMemcpyAsync(fano_cycles, d_cyc, (size_t)ncand * sizeof(uint32_t), cudaMemcpyDeviceToHost, cs));
+    CU(cudaStreamSynchronize(cs));
+    int n = 0;
+    for (int g = 0; g < ncand; g++) n += decoded[g];
+    *ndecoded = n;
+    return UWSPR_B200_OK;
+}
+
+int fano_rows_impl(uwspr_b200_ctx *ctx, const uint8_t *symbols, int space, int n, uint32_t nbits, int delta,
+                   uint32_t maxcycles, int32_t *status, uint32_t *metric, uint32_t *cycles, uint32_t *maxnp, uint8_t *data11)
+{
+    CU(cudaSetDevice(ctx->device));
+    int rc = ensure_mettab(ctx);
+    if (rc) return rc;
+    Buffers &b = ctx->b;
+    // symbols, then the four counters and data11, each array 16-byte aligned
+    const size_t m = (size_t)n, sym_bytes = (m * UW_NSYM + 15) & ~(size_t)15, cnt_bytes = (m * sizeof(uint32_t) + 15) & ~(size_t)15;
+    const size_t need = sym_bytes + 4 * cnt_bytes + m * 11;
+    if (need > b.rows_cap) {
+        if (b.rows) cudaFree(b.rows);
+        b.rows = nullptr;
+        b.rows_cap = 0;
+        CU(cudaMalloc(&b.rows, need));
+        b.rows_cap = need;
+    }
+    cudaStream_t cs = ctx->compute;
+    uint8_t *d_sym = b.rows;
+    int32_t *d_status = reinterpret_cast<int32_t *>(b.rows + sym_bytes);
+    uint32_t *d_metric = reinterpret_cast<uint32_t *>(b.rows + sym_bytes + cnt_bytes);
+    uint32_t *d_cycles = reinterpret_cast<uint32_t *>(b.rows + sym_bytes + 2 * cnt_bytes);
+    uint32_t *d_maxnp = reinterpret_cast<uint32_t *>(b.rows + sym_bytes + 3 * cnt_bytes);
+    uint8_t *d_data = b.rows + sym_bytes + 4 * cnt_bytes;
+    const uint8_t *src = symbols;
+    if (space == UWSPR_B200_HOST) {
+        CU(cudaMemcpyAsync(d_sym, symbols, m * UW_NSYM, cudaMemcpyHostToDevice, cs));
+        src = d_sym;
+    }
+    uw_launch_fano_rows(src, n, (int)nbits, delta, maxcycles, b.mettab, d_status, d_metric, d_cycles, d_maxnp, d_data, cs);
+    ctx->launches++;
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(status, d_status, m * sizeof(int32_t), cudaMemcpyDeviceToHost, cs));
+    CU(cudaMemcpyAsync(metric, d_metric, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, cs));
+    CU(cudaMemcpyAsync(cycles, d_cycles, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, cs));
+    CU(cudaMemcpyAsync(maxnp, d_maxnp, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, cs));
+    CU(cudaMemcpyAsync(data11, d_data, m * 11, cudaMemcpyDeviceToHost, cs));
+    CU(cudaStreamSynchronize(cs));
+    return UWSPR_B200_OK;
+}
+
+// as run(): nothing may still run on the context's stream once an error status has been returned
+int settle(uwspr_b200_ctx *ctx, int rc)
+{
+    if (rc != UWSPR_B200_OK) {
+        cudaStreamSynchronize(ctx->compute);
+        cudaGetLastError();
+    }
+    return rc;
+}
+
+}  // namespace
+
+extern "C" {
+
+int uwspr_b200_decode_device(uwspr_b200_ctx *ctx, const uwspr_b200_refined_t *refined, const uwspr_b200_jiggle_t *jig,
+                             const uint8_t *soft, int space, int64_t ncand, int jig_count, uint8_t *decoded,
+                             int8_t *messages7, int32_t *idt_used, uint32_t *fano_cycles)
+{
+    if (!ctx) return -UWSPR_B200_E_PARAM;
+    if (busy(ctx)) return -UWSPR_B200_E_STATE;
+    if (ncand < 0 || jig_count < 0 || jig_count > UWSPR_B200_NJIG)
+        return -fail(ctx, UWSPR_B200_E_PARAM, "ncand < 0 or jig_count outside [0, 17]");
+    if (!refined && !jig && !soft) {
+        if (!ctx->have_fine) return -fail(ctx, UWSPR_B200_E_STATE, "no fine results on the device: call uwspr_b200_fine / coarse_fine first");
+        if (ncand != ctx->last_total || jig_count != ctx->last_jig_count)
+            return -fail(ctx, UWSPR_B200_E_PARAM, "ncand / jig_count differ from the last fine call's candidate total / jiggle count");
+    } else {
+        if (!refined || !jig || !soft) return -fail(ctx, UWSPR_B200_E_PARAM, "refined, jig and soft: all given or all NULL");
+        if (space != UWSPR_B200_HOST && space != UWSPR_B200_DEVICE) return -fail(ctx, UWSPR_B200_E_PARAM, "space must be HOST or DEVICE");
+        if (ncand > ctx->max_candidates) return -fail(ctx, UWSPR_B200_E_CAPACITY, "more candidates than max_candidates");
+    }
+    if (ncand == 0) return 0;
+    if (!decoded || !messages7) return -fail(ctx, UWSPR_B200_E_PARAM, "decoded and messages7 are required");
+    int n = 0;
+    const int rc = settle(ctx, decode_impl(ctx, refined, jig, soft, space, (int)ncand, jig_count, decoded, messages7, idt_used,
+                                           fano_cycles, &n));
+    return rc ? -rc : n;
+}
+
+int uwspr_b200_fano_batch(uwspr_b200_ctx *ctx, const uint8_t *symbols, int space, int64_t n, uint32_t nbits, int delta,
+                          uint32_t maxcycles, int32_t *status, uint32_t *metric, uint32_t *cycles, uint32_t *maxnp,
+                          uint8_t *data11)
+{
+    if (!ctx) return UWSPR_B200_E_PARAM;
+    if (!fano_domain(nbits, delta, maxcycles))
+        return fail(ctx, UWSPR_B200_E_PARAM, "need 32 <= nbits <= 81, delta > 0, maxcycles >= 1 and (maxcycles*nbits + 1)*delta < 2^31");
+    if (n < 0 || n > INT_MAX - 64) return fail(ctx, UWSPR_B200_E_PARAM, "row count out of range");
+    if (space != UWSPR_B200_HOST && space != UWSPR_B200_DEVICE) return fail(ctx, UWSPR_B200_E_PARAM, "space must be HOST or DEVICE");
+    if (busy(ctx)) return UWSPR_B200_E_STATE;
+    if (n == 0) return UWSPR_B200_OK;
+    if (!symbols || !status || !metric || !cycles || !maxnp || !data11) return fail(ctx, UWSPR_B200_E_PARAM, "NULL buffer");
+    return settle(ctx, fano_rows_impl(ctx, symbols, space, (int)n, nbits, delta, maxcycles, status, metric, cycles, maxnp, data11));
 }
 
 int uwspr_b200_host_alloc(void **ptr, size_t bytes)

@@ -135,3 +135,15 @@ size_t uw_coarse_smem_bytes(const UwDims &d);
 int uw_coarse_setup(const UwDims &d);
 int uw_fine_setup();
 int uw_coarse_blocks_per_sm(const UwDims &d);
+// the Fano decoder (fano.cu).  Candidate form: task list, decoder tasks and per-candidate reduction over
+// refined[ncand], jig/soft[ncand][jig_count]; workspaces first_ok[ncand], tasks/task_cycles/task_msg
+// [ncand*jig_count], counters[2]; grid = resident blocks of the decoder kernel.
+void uw_launch_fano_candidates(const uwspr_b200_refined_t *refined, const uwspr_b200_jiggle_t *jig, const uint8_t *soft,
+                               int ncand, int jig_count, const short *mettab, int *first_ok, int *tasks, int *counters,
+                               uint32_t *task_cycles, unsigned long long *task_msg, int grid, uint8_t *decoded,
+                               int8_t *msg7, int32_t *idt_used, uint32_t *fano_cycles, cudaStream_t s);
+// raw form: n rows of 162 de-interleaved symbols -> uwspr_b200_fano's outputs per row
+void uw_launch_fano_rows(const uint8_t *symbols, int n, int nbits, int delta, uint32_t maxcycles, const short *mettab,
+                         int32_t *status, uint32_t *metric, uint32_t *cycles, uint32_t *maxnp, uint8_t *data11, cudaStream_t s);
+int uw_fano_setup();
+int uw_fano_blocks_per_sm();

@@ -181,9 +181,6 @@ receiver::receiver(const uwspr_b200_params_t &fdr_params, int shift_seconds, int
     }
     d_npk.resize(d_batch);
     d_cands.resize(d_cap);
-    d_refined.resize(d_cap);
-    d_jig.resize((size_t)d_cap * UWSPR_B200_NJIG);
-    d_soft.resize((size_t)d_cap * UWSPR_B200_NJIG * UWSPR_B200_NSYM);
 }
 
 receiver::~receiver() { uwspr_b200_destroy(d_ctx); }
@@ -193,16 +190,14 @@ void receiver::run_batch(int nwin)
     int32_t total = 0;
     check(d_ctx, uwspr_b200_coarse_fine(d_ctx, reinterpret_cast<const float *>(d_stream.data()), UWSPR_B200_HOST, d_stride,
                                         nwin, 0, UWSPR_B200_NJIG, d_npk.data(), d_cands.data(), d_cap, &total,
-                                        d_refined.data(), d_jig.data(), d_soft.data()));
-    int ncand = 0;
-    for (int w = 0; w < nwin; w++) ncand += d_npk[w];
-    // the decoder of every candidate of the batch, spread over the host cores; messages are
-    // still published in (window, candidate) order
-    std::vector<uint8_t> decoded((size_t)ncand);
-    std::vector<int8_t> blobs((size_t)ncand * 7);
-    if (uwspr_b200_decode_batch(d_refined.data(), d_jig.data(), d_soft.data(), ncand, UWSPR_B200_NJIG, 0,
-                                decoded.data(), blobs.data(), nullptr, nullptr) < 0)
-        throw context_error(UWSPR_B200_E_PARAM, "uwspr_b200_decode_batch failed");
+                                        nullptr, nullptr, nullptr));
+    // the decoder of every candidate of the batch runs on the device, on the refinement results and
+    // soft symbols the call above left there; messages are still published in (window, candidate) order
+    std::vector<uint8_t> decoded((size_t)total);
+    std::vector<int8_t> blobs((size_t)total * 7);
+    const int got = uwspr_b200_decode_device(d_ctx, nullptr, nullptr, nullptr, UWSPR_B200_DEVICE, total, UWSPR_B200_NJIG,
+                                             decoded.data(), blobs.data(), nullptr, nullptr);
+    if (got < 0) throw context_error(-got, uwspr_b200_last_error(d_ctx));
     int g = 0;
     for (int w = 0; w < nwin; w++)
         for (int j = 0; j < d_npk[w]; j++, g++) {

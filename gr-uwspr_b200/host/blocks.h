@@ -142,9 +142,6 @@ private:
     std::deque<message_pdu> d_msgs;
     std::vector<int32_t> d_npk;
     std::vector<uwspr_b200_candidate_t> d_cands;
-    std::vector<uwspr_b200_refined_t> d_refined;
-    std::vector<uwspr_b200_jiggle_t> d_jig;
-    std::vector<uint8_t> d_soft;
 };
 
 }  // namespace uwspr

@@ -20,6 +20,7 @@ EXPORTED_SYMBOLS = [
     "uwspr_b200_receiver_windows", "uwspr_b200_hashtab_bytes", "uwspr_b200_unpack", "uwspr_b200_format_message_log",
     "uwspr_b200_pack_type1", "uwspr_b200_channel_symbols", "uwspr_b200_read_c2", "uwspr_b200_frontend", "uwspr_b200_frontend_ctaps",
     "uwspr_b200_frontend_error", "uwspr_b200_coarse_fine_submit", "uwspr_b200_poll", "uwspr_b200_wait",
+    "uwspr_b200_decode_device", "uwspr_b200_fano_batch",
 ]
 
 CAND_DTYPE = np.dtype(
@@ -104,6 +105,10 @@ def load_library():
     L.uwspr_b200_decode_candidate.argtypes = [vp, vp, vp, C.c_int, vp, vp, vp]
     L.uwspr_b200_decode_batch.restype = C.c_int
     L.uwspr_b200_decode_batch.argtypes = [vp, vp, vp, C.c_int64, C.c_int, C.c_int, vp, vp, vp, vp]
+    L.uwspr_b200_decode_device.restype = C.c_int
+    L.uwspr_b200_decode_device.argtypes = [vp, vp, vp, vp, C.c_int, C.c_int64, C.c_int, vp, vp, vp, vp]
+    L.uwspr_b200_fano_batch.restype = C.c_int
+    L.uwspr_b200_fano_batch.argtypes = [vp, vp, C.c_int, C.c_int64, C.c_uint32, C.c_int, C.c_uint32, vp, vp, vp, vp, vp]
     L.uwspr_b200_pack_type1.restype = C.c_int
     L.uwspr_b200_pack_type1.argtypes = [C.c_char_p, C.c_char_p, C.c_int, vp]
     L.uwspr_b200_channel_symbols.restype = None
@@ -149,6 +154,16 @@ def _p(a):
     return a.ctypes.data_as(C.c_void_p) if a is not None else None
 
 
+def _buffer_arg(a, dtype):
+    """(pointer, space, keep-alive, byte size) of a numpy array (host) or a contiguous CUDA tensor (device)"""
+    if hasattr(a, "data_ptr") and getattr(a, "is_cuda", False):
+        if not a.is_contiguous():
+            raise ValueError("CUDA tensors must be contiguous")
+        return C.c_void_p(a.data_ptr()), DEVICE, a, a.numel() * a.element_size()
+    h = np.ascontiguousarray(a, dtype=dtype)
+    return _p(h), HOST, h, h.nbytes
+
+
 def _samples_arg(samples):
     """accepts a numpy complex64 array (host) or (device_pointer:int, n_complex:int) for device memory"""
     if isinstance(samples, tuple):
@@ -172,6 +187,8 @@ class Context:
         self.h = h
         self.fl = fl
         self._pinned = []
+        self._fine = None          # (candidate total, jiggle count) of the fine results on the device
+        self._coarse_total = 0     # candidates of the list on the device
         inf = Info()
         self._check(self.L.uwspr_b200_info(self.h, C.byref(inf)))
         self.info = inf
@@ -218,6 +235,8 @@ class Context:
         cands = np.zeros(cap, CAND_DTYPE) if fetch else None
         total = C.c_int32(0)
         self._check(self.L.uwspr_b200_coarse(self.h, ptr, space, stride, nwin, _p(npk), _p(cands), cap, C.byref(total)))
+        self._fine = None
+        self._coarse_total = total.value
         if not fetch:
             return total.value
         return npk, cands[: total.value].copy()
@@ -239,6 +258,7 @@ class Context:
         soft = np.zeros((n_out, jig_count, NSYM), np.uint8) if fetch else None
         self._check(self.L.uwspr_b200_fine(self.h, ptr, space, stride, nwin, _p(npk), _p(cands), total, jig_first,
                                            jig_count, _p(refined), _p(jig), _p(soft)))
+        self._fine = (total if cands is not None else self._coarse_total, jig_count)
         return refined, jig, soft
 
     def result_buffers(self, nwin, jig_count=NJIG, pinned=True):
@@ -271,6 +291,8 @@ class Context:
         if not fetch:
             self._check(self.L.uwspr_b200_coarse_fine(self.h, ptr, space, stride, nwin, jig_first, jig_count, None, None,
                                                       0, C.byref(total), None, None, None))
+            self._fine = (total.value, jig_count)
+            self._coarse_total = total.value
             return total.value
         if out is not None:
             # views into the caller's buffers, no copies
@@ -278,6 +300,8 @@ class Context:
                                                       _p(out["npk"]), _p(out["cands"]), cap, C.byref(total),
                                                       _p(out["refined"]), _p(out["jig"]), _p(out["soft"])))
             t = total.value
+            self._fine = (t, jig_count)
+            self._coarse_total = t
             return out["npk"][:nwin], out["cands"][:t], out["refined"][:t], out["jig"][:t], out["soft"][:t]
         npk = np.zeros(nwin, np.int32)
         cands = np.zeros(cap, CAND_DTYPE)
@@ -287,6 +311,8 @@ class Context:
         self._check(self.L.uwspr_b200_coarse_fine(self.h, ptr, space, stride, nwin, jig_first, jig_count, _p(npk),
                                                   _p(cands), cap, C.byref(total), _p(refined), _p(jig), _p(soft)))
         t = total.value
+        self._fine = (t, jig_count)
+        self._coarse_total = t
         return npk, cands[:t].copy(), refined[:t].copy(), jig[:t].copy(), soft[:t].copy()
 
     def submit(self, samples, out, nwin=None, stride=None, jig_first=0, jig_count=NJIG):
@@ -296,7 +322,7 @@ class Context:
         ptr, space, keep = _samples_arg(samples)
         nwin = self._nwin(samples, nwin, stride) if not isinstance(samples, tuple) else nwin
         total = C.c_int32(0)
-        self._pending = (keep, out, nwin, total)
+        self._pending = (keep, out, nwin, total, jig_count)
         self._check(self.L.uwspr_b200_coarse_fine_submit(self.h, ptr, space, stride, nwin, jig_first, jig_count, _p(out["npk"]),
                                                          _p(out["cands"]), self.info.max_candidates, C.byref(total),
                                                          _p(out["refined"]), _p(out["jig"]), _p(out["soft"])))
@@ -305,11 +331,42 @@ class Context:
         return int(self.L.uwspr_b200_poll(self.h))
 
     def wait(self):
-        keep, out, nwin, total = self._pending
+        keep, out, nwin, total, jig_count = self._pending
         self._check(self.L.uwspr_b200_wait(self.h))
         self._pending = None
         t = total.value
+        self._fine = (t, jig_count)
+        self._coarse_total = t
         return out["npk"][:nwin], out["cands"][:t], out["refined"][:t], out["jig"][:t], out["soft"][:t]
+
+    # ---- the decoder on the device ---------------------------------------------------------
+    def decode(self, refined=None, jig=None, soft=None, jig_count=NJIG, cycles=False):
+        """uwspr_b200_decode_device: the list decode_candidates() returns -- (candidate index, 7-byte message, idt
+        used) per decoded candidate, in candidate order -- and with cycles=True also the decoder cycles of every
+        candidate (a uint32 array), as (list, cycles).  Without inputs it decodes the results the last fine /
+        coarse_fine call left on the device (jig_count must be that call's); otherwise refined [n], jig [n, jig_count]
+        and soft [n, jig_count, 162] are numpy arrays (host) or contiguous CUDA tensors holding the same bytes."""
+        if refined is None and jig is None and soft is None:
+            ncand = self._fine[0] if self._fine else 0
+            args, space = (None, None, None), HOST
+        else:
+            r, space, kr, nbytes = _buffer_arg(refined, REFINED_DTYPE)
+            j, sj, kj, _ = _buffer_arg(jig, JIG_DTYPE)
+            s, ss, ks, _ = _buffer_arg(soft, np.uint8)
+            if not space == sj == ss:
+                raise ValueError("refined, jig and soft must all be on the host or all on the device")
+            ncand = nbytes // REFINED_DTYPE.itemsize
+            args = (r, j, s)
+        n = max(ncand, 1)
+        decoded = np.zeros(n, np.uint8)
+        msgs = np.zeros((n, 7), np.int8)
+        idt = np.zeros(n, np.int32)
+        cyc = np.zeros(n, np.uint32)
+        got = self.L.uwspr_b200_decode_device(self.h, *args, space, ncand, jig_count, _p(decoded), _p(msgs), _p(idt), _p(cyc))
+        if got < 0:
+            self._check(-got)
+        out = [(int(g), msgs[g].view(np.uint8).copy(), int(idt[g])) for g in np.flatnonzero(decoded[:ncand])]
+        return (out, cyc[:ncand].copy()) if cycles else out
 
     def debug_spectrogram(self, win=0):
         ps = np.zeros((self.info.n_rows, self.info.n_bins), np.float32)
@@ -338,6 +395,20 @@ def fano(symbols, delta=60, maxcycles=10000, nbits=81):
     metric, cycles, maxnp = C.c_uint32(), C.c_uint32(), C.c_uint32()
     r = load_library().uwspr_b200_fano(C.byref(metric), C.byref(cycles), C.byref(maxnp), _p(data), _p(s), nbits, delta, maxcycles)
     return r, data, metric.value, cycles.value, maxnp.value
+
+
+def fano_batch(ctx, symbols, delta=60, maxcycles=10000, nbits=81):
+    """uwspr_b200_fano_batch: fano() on every row of symbols [n, 162] (de-interleaved; numpy or a CUDA tensor) on
+    ctx's device.  Returns arrays mirroring fano()'s tuple: status [n] (0 / -1), data [n, 11], metric, cycles,
+    maxnp [n]."""
+    ptr, space, keep, nbytes = _buffer_arg(symbols, np.uint8)
+    n = nbytes // NSYM
+    status = np.zeros(n, np.int32)
+    data = np.zeros((n, 11), np.uint8)
+    metric, cycles, maxnp = (np.zeros(n, np.uint32) for _ in range(3))
+    ctx._check(ctx.L.uwspr_b200_fano_batch(ctx.h, ptr, space, n, nbits, delta, maxcycles, _p(status), _p(metric),
+                                           _p(cycles), _p(maxnp), _p(data)))
+    return status, data, metric, cycles, maxnp
 
 
 def decode_candidates(refined, jig, soft, nthreads=0):

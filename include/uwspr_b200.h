@@ -207,6 +207,30 @@ UWSPR_B200_API int uwspr_b200_decode_batch(const uwspr_b200_refined_t *refined,
                                            uint8_t *decoded, int8_t *messages7, int32_t *idt_used,
                                            uint32_t *fano_cycles);
 
+/* ---- the same decoder on the device (sm_100a; bit-identical to the two host entry points above) ------
+ * uwspr_b200_decode_device: uwspr_b200_decode_batch's loop with every gated (candidate, jiggle) decoded by
+ * its own device thread; same outputs (host pointers; idt_used and fano_cycles may be NULL) and the same
+ * return value: the number of decoded candidates, or a negative status.
+ * refined == jig == soft == NULL: decodes the results the last uwspr_b200_fine / uwspr_b200_coarse_fine call
+ * on this context left on the device (so a coarse_fine(..., soft = NULL) never copies soft symbols to the
+ * host); ncand and jig_count must equal that call's candidate total and jiggle count (else E_PARAM), and
+ * E_STATE if no such results exist.  Otherwise the three inputs are read from `space` (HOST or DEVICE);
+ * they are copied into the context's device result buffers, which replaces the results of the last call,
+ * and more than max_candidates is E_CAPACITY.  E_STATE while a submission is outstanding.  Runs on the
+ * stream of uwspr_b200_set_stream. */
+UWSPR_B200_API int uwspr_b200_decode_device(uwspr_b200_ctx *ctx, const uwspr_b200_refined_t *refined,
+                                            const uwspr_b200_jiggle_t *jig, const uint8_t *soft, int space,
+                                            int64_t ncand, int jig_count, uint8_t *decoded, int8_t *messages7,
+                                            int32_t *idt_used, uint32_t *fano_cycles);
+/* uwspr_b200_fano on n independent rows of 162 de-interleaved symbols (symbols[n*162] in `space`), one
+ * device thread each; every output (host pointers, n entries; data11: n x 11 bytes, zero past nbits/8)
+ * equals uwspr_b200_fano's for that row, the partial path of a time-out included.  Domain:
+ * 32 <= nbits <= 81, delta > 0, maxcycles >= 1 and (maxcycles*nbits + 1)*delta < 2^31; outside it, or with
+ * a NULL ctx, E_PARAM before any CUDA call.  Returns a status. */
+UWSPR_B200_API int uwspr_b200_fano_batch(uwspr_b200_ctx *ctx, const uint8_t *symbols, int space, int64_t n,
+                                         uint32_t nbits, int delta, uint32_t maxcycles, int32_t *status,
+                                         uint32_t *metric, uint32_t *cycles, uint32_t *maxnp, uint8_t *data11);
+
 /* ---- WSPR_unpacker's text: lib/helpers.cc:494-590 (unpk_) -------------------------------
  * message7 -> "CALL GRID dBm" (type 1), "PFX/CALL dBm" (type 2) or "<CALL> GRID6 dBm" (type 3).
  * hashtab: caller-owned callsign hash table of uwspr_b200_hashtab_bytes() zero-initialised
@@ -261,7 +285,8 @@ UWSPR_B200_API int uwspr_b200_format_message_log(int framecount, const uwspr_b20
 /* ---- batched receive chain of one stream (one hydrophone channel) -----------------------
  * The sliding window of lib/sliding_window_stream_to_pdu_impl.cc:98-138 (window k =
  * stream[k*shift*fs, k*shift*fs + fl)) feeding the device `batch_windows` windows per
- * submission as one contiguous span + stride, then the host-side decode loop.  Messages come
+ * submission as one contiguous span + stride, then the decoder on the device
+ * (uwspr_b200_decode_device on the results left there; no soft symbol crosses PCIe).  Messages come
  * out in (window, candidate) order, one per decoded candidate, no de-duplication -- as the
  * reference publishes them. */
 typedef struct uwspr_b200_receiver uwspr_b200_receiver;
