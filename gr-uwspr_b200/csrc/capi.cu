@@ -309,8 +309,8 @@ int ensure_stage(uwspr_b200_ctx *ctx, size_t elems)
 //   do_coarse: spectrogram + normalizer + peaks + coarse search -> device candidate list
 //   do_fine:   refinement + soft symbols for the device candidate list
 // When !do_coarse the candidate list (npk + cands) is uploaded from the caller first.
-int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_stride, int nwin, bool do_coarse,
-             bool do_fine, const int32_t *npk_in, const uwspr_b200_candidate_t *cands_in, int total_in, int jig_first,
+int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_stride, int wins_per_chan,
+             int64_t chan_stride, int nwin, bool do_coarse, bool do_fine, const int32_t *npk_in, const uwspr_b200_candidate_t *cands_in, int total_in, int jig_first,
              int jig_count, int32_t *npk_out, uwspr_b200_candidate_t *cands_out, int cap_out, int32_t *total_out,
              uwspr_b200_refined_t *refined_out, uwspr_b200_jiggle_t *jig_out, uint8_t *soft_out)
 {
@@ -370,9 +370,15 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
         if (!host || kn.no_tail_split) tail_groups = 0;
         const int ngroups = (nwin + cw - 1) / cw;
         int w = 0, cset = nsets, rr = 0;
-        for (int group = 0; group < ngroups; group++) {
-            const int gw = std::min(cw, nwin - w), set = group % nsets;
-            const bool cut = group > 0 && group >= ngroups - tail_groups && gw > piece;
+        for (int group = 0; w < nwin; group++) {
+            int gw = std::min(cw, nwin - w);
+            const int set = group % nsets;
+            if (!host) {
+                // the fine path keeps window offsets from the chunk's first window in 32 bits (uw_window_offset)
+                const UwGeom g{ (long long)win_stride, (long long)chan_stride, wins_per_chan, w };
+                while (gw > 1 && uw_window_offset(g, gw - 1) - uw_window_offset(g, 0) > INT_MAX) gw = (gw + 1) / 2;
+            }
+            const bool cut = host && group > 0 && group >= ngroups - tail_groups && gw > piece;
             if (!cut) {
                 chunks.push_back(UwChunk{ w, gw, set, 0, set, group, set, 0 });
                 w += gw;
@@ -445,7 +451,10 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
         const int w0 = ch.w0, nw = ch.nw, s = ch.set;
         const bool first_of_group = c == 0 || chunks[c - 1].group != ch.group;
         cudaStream_t st = streams[ch.strm];
+        // window w of the chunk is window ch.w0 + w of the call: staged host input holds only the chunk's windows
+        // (one channel), device input is addressed from the call's first sample
         const float2 *xdev;
+        UwGeom geom{ (long long)win_stride, (long long)chan_stride, wins_per_chan, w0 };
         if (host) {
             // copy stream: wait until the kernels of the chunk two groups back released this buffer
             // set, then copy
@@ -458,9 +467,12 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
             if (ctx->knobs.trace && c == nchunks - 1) CU(cudaEventRecord(ctx->ev_cp1, ctx->copy));
             CU(cudaStreamWaitEvent(st, ctx->ev_h2d[s], 0));
             xdev = b.x_stage[s] + ch.xoff;
+            geom = UwGeom{ (long long)win_stride, 0, nw, 0 };
         } else {
-            xdev = reinterpret_cast<const float2 *>(samples) + (size_t)w0 * (size_t)win_stride;
+            xdev = reinterpret_cast<const float2 *>(samples);
         }
+        // the fine path addresses its windows from the chunk's first one (32-bit offsets)
+        const float2 *xfine = xdev + uw_window_offset(geom, 0);
         // per-set slices of the chunk buffers
         const size_t so = (size_t)s * cw + (size_t)ch.slot;
         float *amp = b.amp + so * d.n_rows * d.nbp;
@@ -471,7 +483,7 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
         cudaEvent_t *e = &ctx->ev[4 * c];
         CU(cudaEventRecord(e[0], st));
         if (do_coarse) {
-            uw_launch_spectrogram(d, xdev, (long long)win_stride, nw, b.window, b.twiddle, amp, psd, psavg, peaks,
+            uw_launch_spectrogram(d, xdev, geom, nw, b.window, b.twiddle, amp, psd, psavg, peaks,
                                   b.npk + w0, st);
             ctx->launches++;
         }
@@ -494,7 +506,7 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
             const long long most = std::min<long long>(ctx->max_candidates, (long long)nw * d.maxcand);
             const int slice = ctx->fine_slice[ch.strm];
             for (long long s0 = 0; s0 < most; s0 += slice)
-                ctx->launches += uw_launch_fine(d, xdev, (long long)win_stride, b.items, set + 1, set + 2, ctx->max_candidates, b.cands,
+                ctx->launches += uw_launch_fine(d, xfine, geom, b.items, set + 1, set + 2, ctx->max_candidates, b.cands,
                                                 jig_first, jig_count, b.refined, b.jig, b.soft, (int)s0, slice,
                                                 b.fine_state[ch.strm], b.fine_pbuf[ch.strm], b.fine_pe[ch.strm], b.fine_pbest[ch.strm], b.fine_tables[ch.strm], b.fine_tickets + 16 * ch.strm, ctx->grid_points,
                                                 ctx->grid_lags, kn.no_fine_reuse ? 0 : 1, st);
@@ -602,9 +614,12 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
 int run(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_stride, int nwin, bool do_coarse,
         bool do_fine, const int32_t *npk_in, const uwspr_b200_candidate_t *cands_in, int total_in, int jig_first,
         int jig_count, int32_t *npk_out, uwspr_b200_candidate_t *cands_out, int cap_out, int32_t *total_out,
-        uwspr_b200_refined_t *refined_out, uwspr_b200_jiggle_t *jig_out, uint8_t *soft_out)
+        uwspr_b200_refined_t *refined_out, uwspr_b200_jiggle_t *jig_out, uint8_t *soft_out, int wins_per_chan = 0,
+        int64_t chan_stride = 0)
 {
-    const int rc = run_impl(ctx, samples, space, win_stride, nwin, do_coarse, do_fine, npk_in, cands_in, total_in, jig_first,
+    // the public entry points pass one stream: every window of the call belongs to channel 0
+    if (wins_per_chan <= 0) wins_per_chan = std::max(nwin, 1);
+    const int rc = run_impl(ctx, samples, space, win_stride, wins_per_chan, chan_stride, nwin, do_coarse, do_fine, npk_in, cands_in, total_in, jig_first,
                             jig_count, npk_out, cands_out, cap_out, total_out, refined_out, jig_out, soft_out);
     if (rc != UWSPR_B200_OK && ctx) {
         cudaStream_t all[5] = { ctx->compute, ctx->compute2, ctx->compute3, ctx->copy, ctx->d2h };
@@ -859,6 +874,23 @@ int uwspr_b200_coarse_fine(uwspr_b200_ctx *ctx, const float *samples, int space,
     return run(ctx, samples, space, win_stride, nwin, true, true, nullptr, nullptr, 0, jig_first, jig_count, npk, cands,
                cap, total, refined, jig, soft);
 }
+
+}  // extern "C"
+
+int uw_coarse_fine_channels(uwspr_b200_ctx *ctx, const float *samples, int64_t win_stride, int wins_per_chan,
+                            int64_t chan_stride, int nchan, int jig_first, int jig_count, int32_t *npk,
+                            uwspr_b200_candidate_t *cands, int cap, int32_t *total)
+{
+    if (!ctx) return UWSPR_B200_E_PARAM;
+    if (busy(ctx)) return UWSPR_B200_E_STATE;
+    if (wins_per_chan < 1 || nchan < 1 || (long long)wins_per_chan * nchan > INT_MAX ||
+        (nchan > 1 && chan_stride < (wins_per_chan - 1) * win_stride + ctx->d.fl))
+        return fail(ctx, UWSPR_B200_E_PARAM, "bad channel geometry");
+    return run(ctx, samples, UWSPR_B200_DEVICE, win_stride, wins_per_chan * nchan, true, true, nullptr, nullptr, 0, jig_first,
+               jig_count, npk, cands, cap, total, nullptr, nullptr, nullptr, wins_per_chan, chan_stride);
+}
+
+extern "C" {
 
 int uwspr_b200_coarse_fine_submit(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_stride, int nwin,
                                   int jig_first, int jig_count, int32_t *npk, uwspr_b200_candidate_t *cands, int cap,

@@ -45,6 +45,24 @@ struct UwPeak {
     float freq, snr;
 };
 
+// Where the windows of one launch live.  Window w of the launch is window W = w0 + w of the call;
+// the call's windows are channel-major, per_chan per channel: window W = c*per_chan + k starts at
+//     x + c*chan_stride + k*win_stride,  x = the call's first sample.
+// A single stream is one channel (per_chan >= the call's window count, chan_stride unused).
+struct UwGeom {
+    long long win_stride, chan_stride;
+    int per_chan, w0;
+};
+
+// offset, in samples from the call's first sample, of window w of the launch; non-decreasing in w when
+// chan_stride >= (per_chan - 1)*win_stride
+__host__ __device__ __forceinline__ long long uw_window_offset(const UwGeom &g, int w)
+{
+    const int W = g.w0 + w;
+    const int c = W / g.per_chan;
+    return (long long)c * g.chan_stride + (long long)(W - c * g.per_chan) * g.win_stride;
+}
+
 __device__ __forceinline__ int uw_sync_bit(const uint32_t *words, int i)
 {
     return (int)((words[i >> 5] >> (i & 31)) & 1u);
@@ -111,7 +129,7 @@ __device__ __forceinline__ uw_f2 uw_fma2(uw_f2 a, uw_f2 b, uw_f2 c)
 __device__ __forceinline__ uw_f2 uw_mul2s(float a, uw_f2 b, uw_f2 nz) { return uw_mul2(uw_pk(a, a), b, nz); }
 
 // launches (defined in the .cu files)
-void uw_launch_spectrogram(const UwDims &d, const float2 *x, long long win_stride, int nwin,
+void uw_launch_spectrogram(const UwDims &d, const float2 *x, const UwGeom &geom, int nwin,
                            const float *window, const float2 *twiddle, float *amp, float *ps_dbg,
                            float *psavg, UwPeak *peaks, int *npk, cudaStream_t s);
 void uw_launch_worklist(const int *npk, int nwin, int cap, int *base, UwItem *items, int *counters,
@@ -120,12 +138,20 @@ void uw_launch_coarse(const UwDims &d, const float *amp, const UwPeak *peaks, co
                       const int *total, int cap, const uint32_t *off4, const short *hyp_unique,
                       uwspr_b200_candidate_t *cands, int *ticket, int grid, cudaStream_t s);
 // the stage sequence of the fine path over work-list entries *begin + slice0 + [0, slice_n); returns the launches issued
-int uw_launch_fine(const UwDims &d, const float2 *x, long long win_stride, const UwItem *items, const int *begin,
+int uw_launch_fine(const UwDims &d, const float2 *x, const UwGeom &geom, const UwItem *items, const int *begin,
                    const int *end, int cap, const uwspr_b200_candidate_t *cands, int jig_first, int jig_count,
                    uwspr_b200_refined_t *refined, uwspr_b200_jiggle_t *jig, uint8_t *soft, int slice0, int slice_n,
                    void *state, void *pbuf, void *pE, void *pbest, void *tables, int *tickets, int grid_points, int grid_lags,
                    int reuse, cudaStream_t s);
-size_t uw_fine_state_bytes();   // per candidate of a slice: chain state, stage magnitudes, jiggle magnitudes
+// uwspr_b200_coarse_fine over nchan channels of device-resident samples, wins_per_chan windows each (window
+// c*wins_per_chan + k at samples + 2*(c*chan_stride + k*win_stride) floats), all jiggles' results left on the device
+// for uwspr_b200_decode_device; npk / cands are host outputs in that channel-major window order (capi.cu)
+int uw_coarse_fine_channels(uwspr_b200_ctx *ctx, const float *samples, int64_t win_stride, int wins_per_chan,
+                            int64_t chan_stride, int nchan, int jig_first, int jig_count, int32_t *npk,
+                            uwspr_b200_candidate_t *cands, int cap, int32_t *total);
+// kernel launches a front-end stream has issued (frontend.cu)
+int64_t uw_frontend_stream_launches(const uwspr_b200_frontend_stream *s);
+size_t uw_fine_state_bytes();  // per candidate of a slice: chain state, stage magnitudes, jiggle magnitudes
 size_t uw_fine_pbuf_bytes();
 size_t uw_fine_pe_bytes();
 size_t uw_fine_pbest_bytes();

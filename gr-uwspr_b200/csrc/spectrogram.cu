@@ -123,7 +123,7 @@ struct __align__(16) SpecSmem {
 // FULL: the row count is a multiple of the four groups (348 = 4 x 87 for the reference's frame length), no row tests
 template <bool FULL>
 __global__ void __launch_bounds__(kThreads, 4)
-k_spectrogram(UwDims d, const float2 *__restrict__ x, long long win_stride, int nwin,
+k_spectrogram(UwDims d, const float2 *__restrict__ x, UwGeom geom, int nwin,
               const float *__restrict__ window, const float2 *__restrict__ twiddle,
               float *__restrict__ amp, float *__restrict__ ps_dbg, float *__restrict__ psavg_out,
               UwPeak *__restrict__ peaks_out, int *__restrict__ npk_out)
@@ -134,7 +134,7 @@ k_spectrogram(UwDims d, const float2 *__restrict__ x, long long win_stride, int 
     const int g = tid >> 6, j = tid & 63;
     const int win = blockIdx.x;
     if (win >= nwin) return;
-    const float2 *xw = x + (long long)win * win_stride;
+    const float2 *xw = x + uw_window_offset(geom, win);
 
     // twiddles laid out so that the lanes of a warp read consecutive words (no bank conflicts)
     for (int t = tid; t < 64; t += kThreads) sm.tw1[t >> 3][t & 7] = twiddle[(8 * (t >> 3) * (t & 7)) & (UW_FFT_N - 1)];
@@ -426,7 +426,7 @@ k_worklist(const int *__restrict__ npk, int nwin, int cap, int *__restrict__ bas
 
 }  // namespace
 
-void uw_launch_spectrogram(const UwDims &d, const float2 *x, long long win_stride, int nwin,
+void uw_launch_spectrogram(const UwDims &d, const float2 *x, const UwGeom &geom, int nwin,
                            const float *window, const float2 *twiddle, float *amp, float *ps_dbg,
                            float *psavg, UwPeak *peaks, int *npk, cudaStream_t s)
 {
@@ -437,10 +437,10 @@ void uw_launch_spectrogram(const UwDims &d, const float2 *x, long long win_strid
         attr_set = true;
     }
     if (d.n_rows % kGroups == 0)
-        k_spectrogram<true><<<nwin, kThreads, sizeof(SpecSmem), s>>>(d, x, win_stride, nwin, window, twiddle, amp, ps_dbg, psavg,
+        k_spectrogram<true><<<nwin, kThreads, sizeof(SpecSmem), s>>>(d, x, geom, nwin, window, twiddle, amp, ps_dbg, psavg,
                                                                      peaks, npk);
     else
-        k_spectrogram<false><<<nwin, kThreads, sizeof(SpecSmem), s>>>(d, x, win_stride, nwin, window, twiddle, amp, ps_dbg, psavg,
+        k_spectrogram<false><<<nwin, kThreads, sizeof(SpecSmem), s>>>(d, x, geom, nwin, window, twiddle, amp, ps_dbg, psavg,
                                                                       peaks, npk);
 }
 

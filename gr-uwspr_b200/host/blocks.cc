@@ -1,5 +1,4 @@
-// Host-side mirror of the gr-uwspr blocks around the hot path (see blocks.h) and the C entry
-// points of the batched receiver.
+// Host-side mirror of the gr-uwspr blocks around the hot path (see blocks.h).
 #include "blocks.h"
 
 #include <string.h>
@@ -161,134 +160,10 @@ int sliding_window_stream_to_pdu::work(int noutput_items, const gr_complex *in)
     return noutput_items;
 }
 
-// ---------------------------------------------------------------------- receiver
-receiver::receiver(const uwspr_b200_params_t &fdr_params, int shift_seconds, int batch_windows)
-{
-    uwspr_b200_params_t p = fdr_params;
-    d_batch = std::max(1, batch_windows);
-    p.max_windows = d_batch;
-    d_ctx = make_ctx(p);
-    uwspr_b200_info_t info;
-    uwspr_b200_info(d_ctx, &info);
-    d_cap = info.max_candidates;
-    d_fl = p.fl;
-    d_stride = shift_seconds * p.fs;
-    // the reference's sliding window peeks fl - shift*fs samples after popping shift*fs (it needs shift*fs <= fl
-    // and does not check); a larger stride would also leave fewer than nwin*stride samples to retire after a flush
-    if (d_stride <= 0 || d_stride > d_fl) {
-        uwspr_b200_destroy(d_ctx);
-        throw std::invalid_argument("receiver: need 0 < shift*fs <= fl");
-    }
-    d_npk.resize(d_batch);
-    d_cands.resize(d_cap);
-}
-
-receiver::~receiver() { uwspr_b200_destroy(d_ctx); }
-
-void receiver::run_batch(int nwin)
-{
-    int32_t total = 0;
-    check(d_ctx, uwspr_b200_coarse_fine(d_ctx, reinterpret_cast<const float *>(d_stream.data()), UWSPR_B200_HOST, d_stride,
-                                        nwin, 0, UWSPR_B200_NJIG, d_npk.data(), d_cands.data(), d_cap, &total,
-                                        nullptr, nullptr, nullptr));
-    // the decoder of every candidate of the batch runs on the device, on the refinement results and
-    // soft symbols the call above left there; messages are still published in (window, candidate) order
-    std::vector<uint8_t> decoded((size_t)total);
-    std::vector<int8_t> blobs((size_t)total * 7);
-    const int got = uwspr_b200_decode_device(d_ctx, nullptr, nullptr, nullptr, UWSPR_B200_DEVICE, total, UWSPR_B200_NJIG,
-                                             decoded.data(), blobs.data(), nullptr, nullptr);
-    if (got < 0) throw context_error(-got, uwspr_b200_last_error(d_ctx));
-    int g = 0;
-    for (int w = 0; w < nwin; w++)
-        for (int j = 0; j < d_npk[w]; j++, g++) {
-            if (!decoded[g]) continue;
-            message_pdu m;
-            memcpy(m.blob, &blobs[(size_t)g * 7], 7);
-            m.candidate = d_cands[g];
-            m.window = d_next_window + w;
-            d_msgs.push_back(m);
-        }
-    // window k = stream[k*shift*fs, k*shift*fs + fl): drop what no later window reads
-    d_stream.erase(d_stream.begin(), d_stream.begin() + (size_t)nwin * d_stride);
-    d_next_window += nwin;
-}
-
-void receiver::push(const gr_complex *in, size_t n)
-{
-    d_stream.insert(d_stream.end(), in, in + n);
-    for (;;) {
-        const long have = d_stream.size() >= (size_t)d_fl ? 1 + (long)((d_stream.size() - d_fl) / d_stride) : 0;
-        if (have < d_batch) break;
-        run_batch(d_batch);
-    }
-}
-
-void receiver::flush()
-{
-    while (d_stream.size() >= (size_t)d_fl) {
-        const long have = 1 + (long)((d_stream.size() - d_fl) / d_stride);
-        run_batch((int)std::min<long>(have, d_batch));
-    }
-}
-
-bool receiver::pop(message_pdu &out)
-{
-    if (d_msgs.empty()) return false;
-    out = d_msgs.front();
-    d_msgs.pop_front();
-    return true;
-}
-
 }  // namespace uwspr
 }  // namespace gr
 
-// ------------------------------------------------------------------ C entry points
-using gr::uwspr::receiver;
-
 extern "C" {
-
-int uwspr_b200_receiver_create(const uwspr_b200_params_t *params, int shift_seconds, int batch_windows,
-                               uwspr_b200_receiver **out)
-{
-    if (!params || !out) return UWSPR_B200_E_PARAM;
-    *out = nullptr;
-    try {
-        *out = reinterpret_cast<uwspr_b200_receiver *>(new receiver(*params, shift_seconds, batch_windows));
-    } catch (const gr::uwspr::context_error &e) {
-        return e.status;
-    } catch (const std::exception &) {
-        return UWSPR_B200_E_PARAM;
-    }
-    return UWSPR_B200_OK;
-}
-
-void uwspr_b200_receiver_destroy(uwspr_b200_receiver *rx) { delete reinterpret_cast<receiver *>(rx); }
-
-int uwspr_b200_receiver_push(uwspr_b200_receiver *rx, const float *iq, int64_t n_complex, int flush)
-{
-    if (!rx || (n_complex > 0 && !iq)) return UWSPR_B200_E_PARAM;
-    try {
-        receiver *r = reinterpret_cast<receiver *>(rx);
-        if (n_complex > 0) r->push(reinterpret_cast<const gr::uwspr::gr_complex *>(iq), (size_t)n_complex);
-        if (flush) r->flush();
-    } catch (const gr::uwspr::context_error &e) {
-        return e.status;
-    } catch (const std::exception &) {
-        return UWSPR_B200_E_PARAM;
-    }
-    return UWSPR_B200_OK;
-}
-
-int uwspr_b200_receiver_pop(uwspr_b200_receiver *rx, int8_t *message7, int64_t *window, uwspr_b200_candidate_t *cand)
-{
-    if (!rx) return 0;
-    gr::uwspr::message_pdu m;
-    if (!reinterpret_cast<receiver *>(rx)->pop(m)) return 0;
-    if (message7) memcpy(message7, m.blob, 7);
-    if (window) *window = m.window;
-    if (cand) *cand = m.candidate;
-    return 1;
-}
 
 int uwspr_b200_format_message_log(int framecount, const uwspr_b200_candidate_t *cand, const int8_t *message7, char *text,
                                   size_t text_cap)
@@ -298,11 +173,6 @@ int uwspr_b200_format_message_log(int framecount, const uwspr_b200_candidate_t *
     if (s.size() + 1 > text_cap) return UWSPR_B200_E_CAPACITY;
     memcpy(text, s.c_str(), s.size() + 1);
     return UWSPR_B200_OK;
-}
-
-int64_t uwspr_b200_receiver_windows(const uwspr_b200_receiver *rx)
-{
-    return rx ? reinterpret_cast<const receiver *>(rx)->windows_done() : 0;
 }
 
 }  // extern "C"

@@ -11,10 +11,11 @@
 //   gr::uwspr::sliding_window_stream_to_pdu::make(fs, fl, shift, C)
 //        include/uwspr/sliding_window_stream_to_pdu.h:52, work() lib/sliding_window_stream_to_pdu_impl.cc:98-138
 //
-// `receiver` is the batched form north_star asks for: the sliding window hands many
-// overlapping windows (and, with one receiver per channel, many channels) to the device in
-// one submission -- the ring's contiguous span plus a stride, so every sample crosses PCIe
-// once -- and runs the host-side decoder on what comes back.
+// `array_receiver` is the batched form north_star asks for: C channels of audio (or 375-sps samples) go
+// through a front-end stream into a ring on the device, and the sliding window hands every channel's
+// overlapping windows to the device in one submission per batch, decoded where they are.  It owns device
+// memory, so it is defined with the kernels' host code (csrc/receiver.cu); uwspr_b200_receiver_* is the same
+// class with one channel.
 #ifndef UWSPR_B200_HOST_BLOCKS_H
 #define UWSPR_B200_HOST_BLOCKS_H
 
@@ -48,6 +49,7 @@ struct message_pdu {
     int8_t blob[7];
     uwspr_b200_candidate_t candidate;  // not in the reference's PDU; kept for logging
     int64_t window;                    // index of the window it came from (receiver only)
+    int32_t channel = 0;               // channel it came from (receiver only)
 };
 
 // text the reference appends to messagelog.txt for one decoded frame, without the two
@@ -119,29 +121,41 @@ private:
     std::function<void(samples_ptr)> d_out;
 };
 
-// Batched receive chain of one stream (one channel): sliding window -> coarse+fine on the
-// device for up to `batch` windows per submission -> host decoder.
-class receiver
+// Receive chain of nchan channels in lockstep: front-end stream -> ring of 375-sps streams on the device ->
+// one coarse+fine submission per `batch` windows of every channel -> decoder on the device.
+class array_receiver
 {
 public:
-    receiver(const uwspr_b200_params_t &fdr_params, int shift_seconds, int batch_windows);
-    ~receiver();
-    // appends stream samples; runs a submission whenever `batch` complete windows are buffered
-    void push(const gr_complex *in, size_t n);
+    // throws context_error (E_PARAM for the checks of uwspr_b200_array_receiver_create)
+    array_receiver(const uwspr_b200_params_t &params, const uwspr_b200_input_t &input, int nchan, int shift_seconds,
+                   int batch_windows);
+    ~array_receiver();
+    // n samples of every channel, channel c at data + c*chan_stride samples; runs a submission whenever `batch`
+    // complete windows are buffered on every channel
+    void push(const void *data, int space, int64_t chan_stride, int64_t n);
     // processes every complete window still buffered
     void flush();
     bool pop(message_pdu &out);
     int64_t windows_done() const { return d_next_window; }
+    int64_t launch_count() const;
 
 private:
-    void run_batch(int nwin);
+    void release();
+    void process(bool all);
+    void run_batch(int per_chan);
     uwspr_b200_ctx *d_ctx = nullptr;
-    int d_fl, d_stride, d_batch, d_cap;
-    std::vector<gr_complex> d_stream;  // samples from the start of window d_next_window
+    uwspr_b200_frontend_stream *d_fe = nullptr;
+    void *d_stream = nullptr;                // cudaStream_t of the ring copies
+    void *d_ring[2] = { nullptr, nullptr };  // complex64 [nchan][d_pitch]: the ring and the buffer its tail moves to
+    int d_cur = 0;
+    int d_device, d_kind, d_nchan, d_fl, d_stride, d_batch, d_cap, d_decim = 1;
+    int64_t d_pitch = 0, d_fill = 0;         // samples per channel of the ring, and those held (from window d_next_window)
     int64_t d_next_window = 0;
     std::deque<message_pdu> d_msgs;
     std::vector<int32_t> d_npk;
     std::vector<uwspr_b200_candidate_t> d_cands;
+    std::vector<uint8_t> d_decoded;
+    std::vector<int8_t> d_blobs;
 };
 
 }  // namespace uwspr

@@ -10,6 +10,7 @@ in-tree CUDA library and a CUDA device, and fails loudly otherwise.
 """
 from .binding import (  # noqa: F401
     CAND_DTYPE, JIG_DTYPE, REFINED_DTYPE, NJIG, NSYM, Context, FDR, UwsprError, lib_path, load_library,
-    sync_and_demodulate, deinterleave, fano, fano_batch, decode_candidates, EXPORTED_SYMBOLS, Receiver, WSPR_unpacker,
+    sync_and_demodulate, deinterleave, fano, fano_batch, decode_candidates, EXPORTED_SYMBOLS, Receiver, ArrayReceiver, FrontendStream,
+    WSPR_unpacker,
     pack_type1, channel_symbols, format_message_log, read_c2, frontend, lowpass_taps, flowgraph_taps, firdes_low_pass, firdes_band_pass, resampler_taps,
 )

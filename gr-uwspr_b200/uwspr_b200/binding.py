@@ -21,6 +21,10 @@ EXPORTED_SYMBOLS = [
     "uwspr_b200_pack_type1", "uwspr_b200_channel_symbols", "uwspr_b200_read_c2", "uwspr_b200_frontend", "uwspr_b200_frontend_ctaps",
     "uwspr_b200_frontend_error", "uwspr_b200_coarse_fine_submit", "uwspr_b200_poll", "uwspr_b200_wait",
     "uwspr_b200_decode_device", "uwspr_b200_fano_batch",
+    "uwspr_b200_frontend_stream_create", "uwspr_b200_frontend_stream_push", "uwspr_b200_frontend_stream_outputs",
+    "uwspr_b200_frontend_stream_destroy", "uwspr_b200_array_receiver_create", "uwspr_b200_array_receiver_push",
+    "uwspr_b200_array_receiver_pop", "uwspr_b200_array_receiver_windows", "uwspr_b200_array_receiver_launch_count",
+    "uwspr_b200_array_receiver_destroy",
 ]
 
 CAND_DTYPE = np.dtype(
@@ -40,6 +44,11 @@ class Params(C.Structure):
     _fields_ = [(n, C.c_int32) for n in (
         "fs", "fl", "spb", "maxdrift", "maxfreqs", "halfbandwidth", "cf", "threshold",
         "device", "max_windows", "max_candidates", "nonlinear_intended_t")]
+
+
+class Input(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("taps", C.c_void_p), ("ntaps", C.c_int32), ("complex_taps", C.c_int32),
+                ("decim", C.c_int32), ("delay", C.c_int32), ("fc", C.c_double), ("fs_in", C.c_double)]
 
 
 class Info(C.Structure):
@@ -143,6 +152,25 @@ def load_library():
     L.uwspr_b200_receiver_pop.argtypes = [vp, vp, vp, vp]
     L.uwspr_b200_receiver_windows.restype = i64
     L.uwspr_b200_receiver_windows.argtypes = [vp]
+    L.uwspr_b200_frontend_stream_create.restype = C.c_int
+    L.uwspr_b200_frontend_stream_create.argtypes = [C.c_int, C.c_int, C.c_int, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double,
+                                                    C.c_double, C.POINTER(vp)]
+    L.uwspr_b200_frontend_stream_push.restype = C.c_int
+    L.uwspr_b200_frontend_stream_push.argtypes = [vp, vp, C.c_int, i64, i64, vp, C.c_int, i64, i64, C.POINTER(i64)]
+    L.uwspr_b200_frontend_stream_outputs.restype = i64
+    L.uwspr_b200_frontend_stream_outputs.argtypes = [vp]
+    L.uwspr_b200_frontend_stream_destroy.argtypes = [vp]
+    L.uwspr_b200_array_receiver_create.restype = C.c_int
+    L.uwspr_b200_array_receiver_create.argtypes = [C.POINTER(Params), C.POINTER(Input), C.c_int, C.c_int, C.c_int, C.POINTER(vp)]
+    L.uwspr_b200_array_receiver_push.restype = C.c_int
+    L.uwspr_b200_array_receiver_push.argtypes = [vp, vp, C.c_int, i64, i64, C.c_int]
+    L.uwspr_b200_array_receiver_pop.restype = C.c_int
+    L.uwspr_b200_array_receiver_pop.argtypes = [vp, vp, vp, vp, vp]
+    L.uwspr_b200_array_receiver_windows.restype = i64
+    L.uwspr_b200_array_receiver_windows.argtypes = [vp]
+    L.uwspr_b200_array_receiver_launch_count.restype = i64
+    L.uwspr_b200_array_receiver_launch_count.argtypes = [vp]
+    L.uwspr_b200_array_receiver_destroy.argtypes = [vp]
     L.uwspr_b200_hashtab_bytes.restype = C.c_size_t
     L.uwspr_b200_unpack.restype = C.c_int
     L.uwspr_b200_unpack.argtypes = [vp, vp, vp, C.c_size_t]
@@ -594,12 +622,7 @@ def frontend(audio, taps=None, decim=32, fc=1500.0, fs_in=12000.0, delay=None, d
     (device pointer, dtype, shape) tuple; the result is a numpy array, or stays on the device when out_device_ptr is
     given.  delay defaults to the filter's group delay."""
     L = load_library()
-    ctaps = taps is not None and np.iscomplexobj(taps)
-    if ctaps:
-        taps = np.ascontiguousarray(taps, dtype=np.complex64)
-    else:
-        taps = lowpass_taps(fs_in=fs_in) if taps is None else np.ascontiguousarray(taps, dtype=np.float32)
-    delay = (len(taps) - 1) // 2 if delay is None else int(delay)
+    taps, ctaps, delay = _frontend_taps(taps, fs_in, delay)
     if isinstance(audio, tuple):
         ptr, dtype, shape = audio
         space_in = 1
@@ -627,6 +650,149 @@ def frontend(audio, taps=None, decim=32, fc=1500.0, fs_in=12000.0, delay=None, d
         return got.value
     out = out[:, :got.value]
     return out[0] if len(shape) == 1 else out
+
+
+def _frontend_taps(taps, fs_in, delay):
+    """(taps as float32 array, complex?, delay): complex taps go as (re, im) pairs; delay defaults to the group delay"""
+    ctaps = taps is not None and np.iscomplexobj(taps)
+    if ctaps:
+        taps = np.ascontiguousarray(taps, dtype=np.complex64)
+    else:
+        taps = lowpass_taps(fs_in=fs_in) if taps is None else np.ascontiguousarray(taps, dtype=np.float32)
+    delay = (len(taps) - 1) // 2 if delay is None else int(delay)
+    return taps, ctaps, delay
+
+
+def _channels_arg(data, dtype):
+    """(pointer, space, keep-alive, nchan, n per channel, channel stride) of [nchan, n] / [n] samples: a numpy array
+    (converted to dtype) or a (device pointer, dtype, shape) tuple of contiguous device memory"""
+    if isinstance(data, tuple):
+        ptr, dt, shape = data
+        if np.dtype(dt) != np.dtype(dtype):
+            raise ValueError("device samples are %s, expected %s" % (np.dtype(dt), np.dtype(dtype)))
+        nchan, n = (1, shape[0]) if len(shape) == 1 else shape
+        return C.c_void_p(int(ptr.value if isinstance(ptr, C.c_void_p) else ptr)), DEVICE, None, nchan, n, n
+    a = np.ascontiguousarray(data, dtype=dtype)
+    nchan, n = (1, a.shape[0]) if a.ndim == 1 else a.shape
+    return _p(a), HOST, a, nchan, n, n
+
+
+class FrontendStream:
+    """frontend() as a stream (uwspr_b200_frontend_stream): push(audio [nchan, n]) returns the outputs the new samples
+    complete, complex64 [nchan, m]; after N samples in any split they equal frontend() over all N bit for bit.
+    fmt is np.float32 or np.int16 (PCM scaled by 1/32768); complex taps select the _ctaps form."""
+
+    def __init__(self, nchan, taps=None, decim=32, fc=1500.0, fs_in=12000.0, delay=None, fmt=np.float32, device=0):
+        self.L = load_library()
+        self.taps, ctaps, self.delay = _frontend_taps(taps, fs_in, delay)
+        self.nchan, self.decim, self.fmt = nchan, decim, np.dtype(fmt)
+        self.pushed = 0   # samples per channel so far
+        h = C.c_void_p()
+        st = self.L.uwspr_b200_frontend_stream_create(device, nchan, 1 if self.fmt == np.int16 else 0, _p(self.taps), len(self.taps),
+                                                      int(ctaps), decim, self.delay, fc, fs_in, C.byref(h))
+        if st != 0:
+            raise UwsprError(st, self.L.uwspr_b200_frontend_error().decode())
+        self.h = h
+
+    def pending(self, n):
+        """outputs a push of n more samples per channel produces"""
+        N = self.pushed + n
+        return max(0, (N - self.delay + self.decim - 1) // self.decim) - self.outputs()
+
+    def push(self, audio, out_device_ptr=None, out_stride=None):
+        """audio: numpy [nchan, n] / [n] or a (device pointer, dtype, shape) tuple.  Returns complex64 [nchan, m], or
+        m when out_device_ptr is given (the outputs are then written there, channel c at out_stride samples)"""
+        ptr, space, keep, nchan, n, stride = _channels_arg(audio, self.fmt)
+        if nchan != self.nchan:
+            raise ValueError("expected %d channels" % self.nchan)
+        cap = self.pending(n)
+        got = C.c_int64()
+        if out_device_ptr is None:
+            out = np.zeros((nchan, max(cap, 1)), np.complex64)
+            optr, ospace, ostride = _p(out), HOST, max(cap, 1)
+        else:
+            out, optr, ospace = None, C.c_void_p(int(out_device_ptr)), DEVICE
+            ostride = cap if out_stride is None else int(out_stride)
+        st = self.L.uwspr_b200_frontend_stream_push(self.h, ptr, space, stride, n, optr, ospace, ostride, cap, C.byref(got))
+        if st != 0:
+            raise UwsprError(st, self.L.uwspr_b200_frontend_error().decode())
+        self.pushed += n
+        return got.value if out is None else out[:, :got.value]
+
+    def outputs(self):
+        return int(self.L.uwspr_b200_frontend_stream_outputs(self.h))
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.uwspr_b200_frontend_stream_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+_INPUT_KINDS = {"complex64": (0, np.complex64), "float32": (1, np.float32), "int16": (2, np.int16)}
+
+
+class ArrayReceiver:
+    """receive chain of nchan channels in lockstep (uwspr_b200_array_receiver): 375-sps complex64 input, or float32 /
+    int16 audio at fs_in through the front-end stream (taps, decim, fc, delay as for frontend()); sliding windows of
+    `shift` seconds, batch_windows windows of every channel per submission, decoded on the device.
+    push(data [nchan, n], flush) returns [(channel, window, message7, candidate)] in (window, channel, candidate) order."""
+
+    def __init__(self, nchan, fs=375, fl=45000, spb=256, maxdrift=0, maxfreqs=200, halfbandwidth=10, cf=1500, threshold=10,
+                 shift=9, batch_windows=16, input="complex64", taps=None, decim=32, fc=1500.0, fs_in=12000.0, delay=None,
+                 device=0, max_candidates=0):
+        self.L = load_library()
+        kind, self.dtype = _INPUT_KINDS[input]
+        prm = Params(fs, fl, spb, maxdrift, maxfreqs, halfbandwidth, cf, threshold, device, 0, max_candidates, 0)
+        if kind == 0:
+            inp = Input(0, None, 0, 0, 0, 0, 0.0, 0.0)
+        else:
+            self.taps, ctaps, delay = _frontend_taps(taps, fs_in, delay)
+            inp = Input(kind, _p(self.taps), len(self.taps), int(ctaps), decim, delay, fc, fs_in)
+        self.nchan = nchan
+        h = C.c_void_p()
+        st = self.L.uwspr_b200_array_receiver_create(C.byref(prm), C.byref(inp), nchan, shift, batch_windows, C.byref(h))
+        if st != 0:
+            text = self.L.uwspr_b200_create_error().decode() if st == 2 else ""
+            raise UwsprError(st, text or self.L.uwspr_b200_status_string(st).decode())
+        self.h = h
+
+    def push(self, data, flush=False):
+        ptr, space, keep, nchan, n, stride = _channels_arg(data, self.dtype)
+        if nchan != self.nchan:
+            raise ValueError("expected %d channels" % self.nchan)
+        st = self.L.uwspr_b200_array_receiver_push(self.h, ptr, space, stride, n, int(flush))
+        if st != 0:
+            raise UwsprError(st, self.L.uwspr_b200_status_string(st).decode())
+        out = []
+        chan, win = C.c_int32(), C.c_int64()
+        msg = np.zeros(7, np.int8)
+        cand = np.zeros(1, CAND_DTYPE)
+        while self.L.uwspr_b200_array_receiver_pop(self.h, C.byref(chan), C.byref(win), _p(cand), _p(msg)):
+            out.append((chan.value, win.value, msg.view(np.uint8).copy(), cand[0].copy()))
+        return out
+
+    def windows_done(self):
+        return int(self.L.uwspr_b200_array_receiver_windows(self.h))
+
+    def launch_count(self):
+        return int(self.L.uwspr_b200_array_receiver_launch_count(self.h))
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.uwspr_b200_array_receiver_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def pack_type1(call, grid, dbm):

@@ -275,7 +275,32 @@ UWSPR_B200_API int uwspr_b200_frontend_ctaps(int device, const void *audio, int 
                                              const float *taps_iq, int ntaps, int decim, int delay, double fc,
                                              double fs_in, float *out, int space_out, int64_t out_stride,
                                              int64_t *n_out);
+/* text of the last front-end failure (one-shot or stream) on the calling thread */
 UWSPR_B200_API const char *uwspr_b200_frontend_error(void);
+
+/* The front-end as a stream that keeps its state between pushes (audio read in pieces, a GNU Radio work() call
+ * at a time).  After N input samples per channel in total, in any split, the stream has produced exactly the
+ * outputs m with m*decim + delay < N, and each equals, bit for bit, output m of uwspr_b200_frontend (real taps) or
+ * uwspr_b200_frontend_ctaps (complex_taps != 0: taps holds ntaps pairs re, im) run once over any input that holds
+ * those samples.  State per channel: the last ntaps - 1 + decim samples in the input format and the sample count.
+ * create allocates every buffer; a push allocates nothing, runs on a stream owned by the object, works through
+ * its input in pieces of bounded size and returns when its outputs are written.
+ * create: E_PARAM for the arguments uwspr_b200_frontend rejects, and when ntaps + 63*decim samples do not fit
+ * shared memory (a device query).  push: audio holds n_in samples of each of the nchan channels, chan_stride
+ * apart, in `space_in`; the new outputs go to out (complex64, channel c at out + 2*c*out_stride floats) in
+ * `space_out`, *n_out of them per channel; more than out_cap is E_CAPACITY and consumes nothing.  After any other
+ * failure of a push the stream's state is lost: later pushes return E_STATE.  chan_stride < n_in or
+ * out_stride < out_cap is E_PARAM, for one channel too. */
+typedef struct uwspr_b200_frontend_stream uwspr_b200_frontend_stream;
+UWSPR_B200_API int uwspr_b200_frontend_stream_create(int device, int nchan, int fmt, const float *taps, int ntaps,
+                                                     int complex_taps, int decim, int delay, double fc, double fs_in,
+                                                     uwspr_b200_frontend_stream **out);
+UWSPR_B200_API int uwspr_b200_frontend_stream_push(uwspr_b200_frontend_stream *s, const void *audio, int space_in,
+                                                   int64_t chan_stride, int64_t n_in, float *out, int space_out,
+                                                   int64_t out_stride, int64_t out_cap, int64_t *n_out);
+/* outputs produced so far, per channel */
+UWSPR_B200_API int64_t uwspr_b200_frontend_stream_outputs(const uwspr_b200_frontend_stream *s);
+UWSPR_B200_API void uwspr_b200_frontend_stream_destroy(uwspr_b200_frontend_stream *s);
 
 /* The text the reference appends to messagelog.txt for one decoded frame
  * (lib/sync_and_demodulate_impl.cc:508-525), without the two wall-clock lines before it. */
@@ -285,10 +310,9 @@ UWSPR_B200_API int uwspr_b200_format_message_log(int framecount, const uwspr_b20
 /* ---- batched receive chain of one stream (one hydrophone channel) -----------------------
  * The sliding window of lib/sliding_window_stream_to_pdu_impl.cc:98-138 (window k =
  * stream[k*shift*fs, k*shift*fs + fl)) feeding the device `batch_windows` windows per
- * submission as one contiguous span + stride, then the decoder on the device
- * (uwspr_b200_decode_device on the results left there; no soft symbol crosses PCIe).  Messages come
- * out in (window, candidate) order, one per decoded candidate, no de-duplication -- as the
- * reference publishes them. */
+ * submission, then the decoder on the device (uwspr_b200_decode_device on the results left there; no soft
+ * symbol crosses PCIe).  Messages come out in (window, candidate) order, one per decoded candidate, no
+ * de-duplication -- as the reference publishes them.  It is the array receiver below with one channel of kind 0. */
 typedef struct uwspr_b200_receiver uwspr_b200_receiver;
 UWSPR_B200_API int uwspr_b200_receiver_create(const uwspr_b200_params_t *params, int shift_seconds,
                                               int batch_windows, uwspr_b200_receiver **out);
@@ -300,6 +324,44 @@ UWSPR_B200_API int uwspr_b200_receiver_push(uwspr_b200_receiver *rx, const float
 UWSPR_B200_API int uwspr_b200_receiver_pop(uwspr_b200_receiver *rx, int8_t *message7, int64_t *window,
                                            uwspr_b200_candidate_t *cand);
 UWSPR_B200_API int64_t uwspr_b200_receiver_windows(const uwspr_b200_receiver *rx);
+
+/* ---- receive chain of nchan channels in lockstep, from audio or 375-sps samples to messages ---------------
+ * Channel c's stream s_c is its input (kind 0) or the output of a uwspr_b200_frontend_stream over its audio
+ * (kinds 1 and 2).  Window k of channel c is s_c[k*shift*fs, k*shift*fs + fl).  The streams live in a ring on the
+ * device; once batch_windows windows are complete on every channel, one coarse_fine submission covers all
+ * nchan * batch_windows windows (17 jiggles, nothing copied back but the candidate list), then
+ * uwspr_b200_decode_device decodes them where they are.  Messages come out in (window, channel, candidate) order,
+ * one per decoded candidate, without de-duplication, and do not depend on batch_windows or on how the input is
+ * split into pushes.  params->max_windows is ignored (nchan * batch_windows); params->max_candidates as for
+ * uwspr_b200_create. */
+typedef struct {
+    int32_t kind;            /* 0: complex64 at params->fs (no front-end), 1: float32 audio, 2: int16 audio */
+    const float *taps;       /* kinds 1, 2: ntaps real taps, or ntaps (re, im) pairs when complex_taps != 0 */
+    int32_t ntaps, complex_taps, decim, delay;
+    double fc, fs_in;        /* fs_in / decim must equal params->fs */
+} uwspr_b200_input_t;
+typedef struct uwspr_b200_array_receiver uwspr_b200_array_receiver;
+/* E_PARAM before any CUDA call: NULL pointers, nchan < 1, batch_windows < 1, shift*fs outside (0, fl], a bad kind,
+ * and for kinds 1 and 2 ntaps outside 1..16384, decim outside 1..4096, delay < 0 or fs_in / decim != fs.
+ * E_PARAM after a device query: ntaps + 63*decim samples do not fit shared memory.  Otherwise as uwspr_b200_create. */
+UWSPR_B200_API int uwspr_b200_array_receiver_create(const uwspr_b200_params_t *params, const uwspr_b200_input_t *input,
+                                                    int nchan, int shift_seconds, int batch_windows,
+                                                    uwspr_b200_array_receiver **out);
+/* n_per_chan samples of every channel (complex64 for kind 0, else the audio format), channel c at
+ * data + c*chan_stride samples (chan_stride >= n_per_chan, else E_PARAM), in `space`; flush != 0 then processes
+ * every complete window still buffered.
+ * A failing batch returns its status (E_CAPACITY when its candidates exceed max_candidates); the receiver's state
+ * is then lost and later pushes return E_STATE. */
+UWSPR_B200_API int uwspr_b200_array_receiver_push(uwspr_b200_array_receiver *rx, const void *data, int space,
+                                                  int64_t chan_stride, int64_t n_per_chan, int flush);
+/* returns 1 and fills the outputs (any may be NULL) while decoded messages are queued, else 0 */
+UWSPR_B200_API int uwspr_b200_array_receiver_pop(uwspr_b200_array_receiver *rx, int32_t *channel, int64_t *window,
+                                                 uwspr_b200_candidate_t *cand, int8_t *message7);
+/* windows processed per channel */
+UWSPR_B200_API int64_t uwspr_b200_array_receiver_windows(const uwspr_b200_array_receiver *rx);
+/* kernel launches issued so far (front-end, search and decoder) */
+UWSPR_B200_API int64_t uwspr_b200_array_receiver_launch_count(const uwspr_b200_array_receiver *rx);
+UWSPR_B200_API void uwspr_b200_array_receiver_destroy(uwspr_b200_array_receiver *rx);
 
 /* ---- utilities ------------------------------------------------------------------------- */
 /* pinned host memory for sample / result buffers (cudaHostAlloc / cudaFreeHost) */
