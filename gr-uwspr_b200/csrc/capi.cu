@@ -47,6 +47,7 @@ struct Knobs {
     bool no_early_d2h = false;  // UWSPR_B200_NO_EARLY_D2H
     bool trace = false;         // UWSPR_B200_TRACE
     bool no_fine_reuse = false; // UWSPR_B200_NO_FINE_REUSE: stage E evaluates jiggle 0 again instead of taking it from the chain
+    bool no_lag_share = false;  // UWSPR_B200_NO_LAG_SHARE: the lag searches (stages A, D) rotate one table set per point (R1)
     int dev_chunks = 1;         // UWSPR_B200_DEV_CHUNKS
     int fine_ctas_per_sm = 0;   // UWSPR_B200_FINE_CTAS_PER_SM: fewer resident CTAs than fit (occupancy experiments)
     int fine_slice = 16384;     // UWSPR_B200_FINE_SLICE: candidates per pass of the fine path's stage sequence
@@ -68,6 +69,7 @@ Knobs read_knobs()
     k.no_early_d2h = getenv("UWSPR_B200_NO_EARLY_D2H") != nullptr;
     k.trace = getenv("UWSPR_B200_TRACE") != nullptr;
     k.no_fine_reuse = getenv("UWSPR_B200_NO_FINE_REUSE") != nullptr;
+    k.no_lag_share = getenv("UWSPR_B200_NO_LAG_SHARE") != nullptr;
     k.dev_chunks = std::max(1, geti("UWSPR_B200_DEV_CHUNKS", 1));
     k.fine_ctas_per_sm = std::max(0, geti("UWSPR_B200_FINE_CTAS_PER_SM", 0));
     k.fine_slice = std::max(1, geti("UWSPR_B200_FINE_SLICE", k.fine_slice));
@@ -126,7 +128,7 @@ struct uwspr_b200_ctx {
     Buffers b;
     int device = 0, sm_count = 0;
     int chunk_windows = 0, max_windows = 0, max_candidates = 0;
-    int grid_coarse = 0, grid_points = 0, grid_lags = 0;
+    int grid_coarse = 0, grid_points = 0, grid_lags = 0, grid_share = 0;
     int fine_slice[3] = { 0, 0, 0 };   // candidates the fine path's stage sequence handles per pass, per compute stream
     cudaStream_t compute = nullptr, compute2 = nullptr, compute3 = nullptr, copy = nullptr, d2h = nullptr;
     int *h_ends = nullptr;  // pinned: end of every chunk's items (host-fed calls stream results back per chunk)
@@ -509,7 +511,7 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
                 ctx->launches += uw_launch_fine(d, xfine, geom, b.items, set + 1, set + 2, ctx->max_candidates, b.cands,
                                                 jig_first, jig_count, b.refined, b.jig, b.soft, (int)s0, slice,
                                                 b.fine_state[ch.strm], b.fine_pbuf[ch.strm], b.fine_pe[ch.strm], b.fine_pbest[ch.strm], b.fine_tables[ch.strm], b.fine_tickets + 16 * ch.strm, ctx->grid_points,
-                                                ctx->grid_lags, kn.no_fine_reuse ? 0 : 1, st);
+                                                ctx->grid_lags, ctx->grid_share, kn.no_fine_reuse ? 0 : 1, st);
         }
         CU(cudaEventRecord(e[3], st));
         if (host) CU(cudaEventRecord(ctx->ev_free[s], st));
@@ -768,17 +770,19 @@ int uwspr_b200_create(const uwspr_b200_params_t *params, uwspr_b200_ctx **ctx_ou
     ctx->grid_coarse = ctx->sm_count * uw_coarse_blocks_per_sm(d);
     ctx->fano_grid = ctx->sm_count * uw_fano_blocks_per_sm();
     {
-        int bp = 1, bl = 1;
-        uw_fine_blocks_per_sm(&bp, &bl);
+        int bp = 1, bl = 1, bs = 1;
+        uw_fine_blocks_per_sm(&bp, &bl, &bs);
         if (ctx->knobs.fine_ctas_per_sm > 0) {
             bp = std::min(bp, ctx->knobs.fine_ctas_per_sm);
             bl = std::min(bl, ctx->knobs.fine_ctas_per_sm);
+            bs = std::min(bs, ctx->knobs.fine_ctas_per_sm);
         }
         ctx->grid_points = ctx->sm_count * bp;
         ctx->grid_lags = ctx->sm_count * bl;
+        ctx->grid_share = ctx->knobs.no_lag_share ? 0 : ctx->sm_count * bs;
         if (ctx->knobs.trace)
-            fprintf(stderr, "uwspr_b200 trace: fine path: %d + %d resident CTAs per SM (points, lags), slices of %d candidates\n", bp, bl,
-                    std::max(1, std::min(ctx->max_candidates, ctx->knobs.fine_slice)));
+            fprintf(stderr, "uwspr_b200 trace: fine path: %d + %d + %d resident CTAs per SM (points, lags, lag share%s), slices of %d candidates\n",
+                    bp, bl, bs, ctx->knobs.no_lag_share ? " off" : "", std::max(1, std::min(ctx->max_candidates, ctx->knobs.fine_slice)));
     }
     CUC(cudaDeviceSynchronize());
 #undef CUC

@@ -137,12 +137,13 @@ void uw_launch_worklist(const int *npk, int nwin, int cap, int *base, UwItem *it
 void uw_launch_coarse(const UwDims &d, const float *amp, const UwPeak *peaks, const UwItem *items,
                       const int *total, int cap, const uint32_t *off4, const short *hyp_unique,
                       uwspr_b200_candidate_t *cands, int *ticket, int grid, cudaStream_t s);
-// the stage sequence of the fine path over work-list entries *begin + slice0 + [0, slice_n); returns the launches issued
+// the stage sequence of the fine path over work-list entries *begin + slice0 + [0, slice_n); returns the launches issued.
+// grid_share: resident CTAs of the lag searches' shared-table kernel, 0 to run the lag searches through R1
 int uw_launch_fine(const UwDims &d, const float2 *x, const UwGeom &geom, const UwItem *items, const int *begin,
                    const int *end, int cap, const uwspr_b200_candidate_t *cands, int jig_first, int jig_count,
                    uwspr_b200_refined_t *refined, uwspr_b200_jiggle_t *jig, uint8_t *soft, int slice0, int slice_n,
                    void *state, void *pbuf, void *pE, void *pbest, void *tables, int *tickets, int grid_points, int grid_lags,
-                   int reuse, cudaStream_t s);
+                   int grid_share, int reuse, cudaStream_t s);
 // uwspr_b200_coarse_fine over nchan channels of device-resident samples, wins_per_chan windows each (window
 // c*wins_per_chan + k at samples + 2*(c*chan_stride + k*win_stride) floats), all jiggles' results left on the device
 // for uwspr_b200_decode_device; npk / cands are host outputs in that channel-major window order (capi.cu)
@@ -156,7 +157,7 @@ size_t uw_fine_pbuf_bytes();
 size_t uw_fine_pe_bytes();
 size_t uw_fine_pbest_bytes();
 size_t uw_fine_tables_bytes();
-void uw_fine_blocks_per_sm(int *points, int *lags);
+void uw_fine_blocks_per_sm(int *points, int *lags, int *share);
 size_t uw_coarse_smem_bytes(const UwDims &d);
 int uw_coarse_setup(const UwDims &d);
 int uw_fine_setup();
