@@ -37,22 +37,14 @@ struct UwChunk {
     size_t xoff;
 };
 
-// Tuning / diagnosis knobs, read from the environment once, when the context is created
+// Test / diagnosis knobs, read from the environment once, when the context is created
 // (DESIGN.md section 3 lists them).
 struct Knobs {
-    int host_chunk = 0;         // UWSPR_B200_HOST_CHUNK: windows per host-fed chunk (0: nwin/16 within [1024, 4096])
     int tail_groups = 2;        // UWSPR_B200_TAIL_GROUPS: chunk groups at the end of a host-fed call that are cut up
     int tail_piece = 0;         // UWSPR_B200_TAIL_PIECE: windows per piece (0: a quarter chunk)
-    bool no_tail_split = false; // UWSPR_B200_NO_TAIL_SPLIT
-    bool no_early_d2h = false;  // UWSPR_B200_NO_EARLY_D2H
     bool trace = false;         // UWSPR_B200_TRACE
     bool no_fine_reuse = false; // UWSPR_B200_NO_FINE_REUSE: stage E evaluates jiggle 0 again instead of taking it from the chain
     bool no_lag_share = false;  // UWSPR_B200_NO_LAG_SHARE: the lag searches (stages A, D) rotate one table set per point (R1)
-    int dev_chunks = 1;         // UWSPR_B200_DEV_CHUNKS
-    int fine_ctas_per_sm = 0;   // UWSPR_B200_FINE_CTAS_PER_SM: fewer resident CTAs than fit (occupancy experiments)
-    int fine_slice = 16384;     // UWSPR_B200_FINE_SLICE: candidates per pass of the fine path's stage sequence
-    int fine_slice_side = 16384; // UWSPR_B200_FINE_SLICE_SIDE: the same for the second and third compute stream (host-fed
-                                // 100 000-window stream: 4096 / 8192 / 16384 -> 247 / 283 / 294 k windows/s)
 };
 
 Knobs read_knobs()
@@ -62,18 +54,11 @@ Knobs read_knobs()
         const char *e = getenv(name);
         return e ? atoi(e) : def;
     };
-    k.host_chunk = std::max(0, geti("UWSPR_B200_HOST_CHUNK", k.host_chunk));
     k.tail_groups = std::max(0, std::min(2, geti("UWSPR_B200_TAIL_GROUPS", k.tail_groups)));
     k.tail_piece = std::max(0, geti("UWSPR_B200_TAIL_PIECE", 0));
-    k.no_tail_split = getenv("UWSPR_B200_NO_TAIL_SPLIT") != nullptr;
-    k.no_early_d2h = getenv("UWSPR_B200_NO_EARLY_D2H") != nullptr;
     k.trace = getenv("UWSPR_B200_TRACE") != nullptr;
     k.no_fine_reuse = getenv("UWSPR_B200_NO_FINE_REUSE") != nullptr;
     k.no_lag_share = getenv("UWSPR_B200_NO_LAG_SHARE") != nullptr;
-    k.dev_chunks = std::max(1, geti("UWSPR_B200_DEV_CHUNKS", 1));
-    k.fine_ctas_per_sm = std::max(0, geti("UWSPR_B200_FINE_CTAS_PER_SM", 0));
-    k.fine_slice = std::max(1, geti("UWSPR_B200_FINE_SLICE", k.fine_slice));
-    k.fine_slice_side = std::max(1, geti("UWSPR_B200_FINE_SLICE_SIDE", k.fine_slice_side));
     return k;
 }
 
@@ -94,13 +79,7 @@ struct Buffers {
     uwspr_b200_refined_t *refined = nullptr;
     uwspr_b200_jiggle_t *jig = nullptr;
     uint8_t *soft = nullptr;
-    int *fine_tickets = nullptr;  // work counters of the fine path's heavy launches, 16 per compute stream
-    // fine path workspaces, one per compute stream (chunks on different streams run concurrently)
-    void *fine_state[3] = { nullptr, nullptr, nullptr };
-    void *fine_pbuf[3] = { nullptr, nullptr, nullptr };
-    void *fine_pe[3] = { nullptr, nullptr, nullptr };
-    void *fine_pbest[3] = { nullptr, nullptr, nullptr };
-    void *fine_tables[3] = { nullptr, nullptr, nullptr };
+    UwFineWork fine[3] = {};  // fine path workspaces, one per compute stream
     int *counters = nullptr;  // [0] running total, [1] overflow; set s at 4+4s: ticket coarse, ticket fine, end of chunk
     // tables
     float *window = nullptr;
@@ -128,8 +107,8 @@ struct uwspr_b200_ctx {
     Buffers b;
     int device = 0, sm_count = 0;
     int chunk_windows = 0, max_windows = 0, max_candidates = 0;
-    int grid_coarse = 0, grid_points = 0, grid_lags = 0, grid_share = 0;
-    int fine_slice[3] = { 0, 0, 0 };   // candidates the fine path's stage sequence handles per pass, per compute stream
+    int grid_coarse = 0;
+    UwFineLaunch fine_launch = {};
     cudaStream_t compute = nullptr, compute2 = nullptr, compute3 = nullptr, copy = nullptr, d2h = nullptr;
     int *h_ends = nullptr;  // pinned: end of every chunk's items (host-fed calls stream results back per chunk)
     bool own_compute = true;
@@ -336,30 +315,22 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
         ctx->last_jig_count = jig_count;
         return UWSPR_B200_OK;
     }
-    // Device-resident input: one stream, chunks as large as the buffers allow (no tails between
-    // chunks).  Host input: chunks of <= 1024 windows alternate between two buffer sets and two
-    // compute streams, so the H2D copy of chunk c+1 and the tail of chunk c-1's kernels overlap
-    // the kernels of chunk c.
+    // Device-resident input: one buffer set and one stream, chunks as large as the buffers allow (no tails between
+    // chunks).  Host input: chunks rotate through three buffer sets and three compute streams, so that the H2D copies
+    // run back to back while earlier chunks are in their kernels.  With two sets the copy of chunk c+2 waited for the
+    // kernels of chunk c, which share the GPU with those of chunk c+1 and take longer than a copy when copy and
+    // compute are balanced (a 100 000-window overlapped stream: 15.2 ms per 4 096-window chunk against 13.3 ms per
+    // copy, trace in profiles/README.md).
     const bool host = space == UWSPR_B200_HOST;
-    // dev_chunks > 1 (tuning knob, UWSPR_B200_DEV_CHUNKS): device input is also split over the two
-    // sets/streams so that one chunk's spectrogram/coarse kernels fill idle issue slots of the
-    // previous chunk's fine kernel
     const Knobs &kn = ctx->knobs;
-    const bool two = host || kn.dev_chunks > 1;
-    // Host input rotates through three buffer sets and three compute streams: with two, the copy of chunk c+2 waited
-    // for the kernels of chunk c, which share the GPU with those of chunk c+1 and take longer than a copy when copy
-    // and compute are balanced (a 100 000-window overlapped stream: 15.2 ms per 4 096-window chunk against 13.3 ms
-    // per copy, trace in profiles/README.md).
-    const int nsets = host ? 3 : (two ? 2 : 1);
+    const int nsets = host ? 3 : 1;
     // host-fed chunk: small enough that the first kernels start early and little is left after the last byte, large
     // enough that the fine path's launches are well filled (measured on a 100 000-window overlapped stream: 1024 /
     // 2048 / 4096 windows per chunk -> 235 / 248 / 251 k windows/s; a 10 000-window call does not care)
-    const int host_chunk = kn.host_chunk > 0 ? kn.host_chunk : std::min(4096, std::max(1024, nwin / 16));
+    const int host_chunk = std::min(4096, std::max(1024, nwin / 16));
     // a call that fits the chunk buffers is cut in three, so that every window's intermediate buffers survive the call
     const int set_cap = nwin <= ctx->chunk_windows ? std::max(ctx->chunk_windows / 3, (nwin + 2) / 3) : ctx->chunk_windows / 3;
-    const int cw = host ? std::max(1, std::min(host_chunk, set_cap))
-                        : (two ? std::max(1, std::min(ctx->chunk_windows / 2, (nwin + kn.dev_chunks - 1) / kn.dev_chunks))
-                               : ctx->chunk_windows);
+    const int cw = host ? std::max(1, std::min(host_chunk, set_cap)) : ctx->chunk_windows;
     // Chunk schedule.  With host input the kernels of a chunk cannot start before its last byte
     // has crossed PCIe, so the end of the call is cut into small pieces (a quarter chunk by
     // default, UWSPR_B200_TAIL_PIECE) that use disjoint slices of their group's buffer set and
@@ -367,9 +338,8 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
     std::vector<UwChunk> &chunks = ctx->last_chunks;
     chunks.clear();
     {
-        int tail_groups = host ? kn.tail_groups : 0;
+        const int tail_groups = host ? kn.tail_groups : 0;
         const int piece = kn.tail_piece > 0 ? kn.tail_piece : std::max(1, cw / 4);
-        if (!host || kn.no_tail_split) tail_groups = 0;
         const int ngroups = (nwin + cw - 1) / cw;
         int w = 0, cset = nsets, rr = 0;
         for (int group = 0; w < nwin; group++) {
@@ -410,7 +380,7 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
         CU(cudaEventCreate(&e));
         ctx->ev.push_back(e);
     }
-    cudaStream_t streams[3] = { cs, two && nchunks > 1 ? ctx->compute2 : cs, ctx->compute3 };
+    cudaStream_t streams[3] = { cs, host && nchunks > 1 ? ctx->compute2 : cs, ctx->compute3 };
     bool use3 = false;
     for (const UwChunk &q : chunks) use3 = use3 || q.strm == 2;
     CU(cudaEventRecord(ctx->ev_begin, cs));
@@ -447,7 +417,7 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
     // Host-fed calls return results chunk by chunk while later chunks are still copying in and
     // computing (PCIe is full duplex); only the last chunk's results are left for the end.
     const bool want_results = (cands_out && do_coarse) || (do_fine && (refined_out || jig_out || soft_out));
-    const bool early = host && nchunks > 1 && want_results && !kn.no_early_d2h;
+    const bool early = host && nchunks > 1 && want_results;
     for (int c = 0; c < nchunks; c++) {
         const UwChunk &ch = chunks[c];
         const int w0 = ch.w0, nw = ch.nw, s = ch.set;
@@ -503,15 +473,14 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
         }
         CU(cudaEventRecord(e[2], st));
         if (do_fine) {
-            // the stage sequence runs over slices of at most fine_slice candidates (the workspace size); the
-            // number of candidates is a device value, so the launches cover the most the chunk can hold
+            // the stage sequence runs over slices of at most the workspace's slice of candidates; the number of
+            // candidates is a device value, so the launches cover the most the chunk can hold
             const long long most = std::min<long long>(ctx->max_candidates, (long long)nw * d.maxcand);
-            const int slice = ctx->fine_slice[ch.strm];
-            for (long long s0 = 0; s0 < most; s0 += slice)
+            const UwFineWork &fw = b.fine[ch.strm];
+            for (long long s0 = 0; s0 < most; s0 += fw.slice)
                 ctx->launches += uw_launch_fine(d, xfine, geom, b.items, set + 1, set + 2, ctx->max_candidates, b.cands,
-                                                jig_first, jig_count, b.refined, b.jig, b.soft, (int)s0, slice,
-                                                b.fine_state[ch.strm], b.fine_pbuf[ch.strm], b.fine_pe[ch.strm], b.fine_pbest[ch.strm], b.fine_tables[ch.strm], b.fine_tickets + 16 * ch.strm, ctx->grid_points,
-                                                ctx->grid_lags, ctx->grid_share, kn.no_fine_reuse ? 0 : 1, st);
+                                                jig_first, jig_count, b.refined, b.jig, b.soft, (int)s0, fw,
+                                                ctx->fine_launch, st);
         }
         CU(cudaEventRecord(e[3], st));
         if (host) CU(cudaEventRecord(ctx->ev_free[s], st));
@@ -718,18 +687,9 @@ int uwspr_b200_create(const uwspr_b200_params_t *params, uwspr_b200_ctx **ctx_ou
     CUC(cudaMalloc(&b.soft, cap * UWSPR_B200_NJIG * UW_NSYM));
     CUC(cudaMalloc(&b.counters, kCounterInts * sizeof(int)));
     CUC(cudaMemset(b.counters, 0, kCounterInts * sizeof(int)));
-    CUC(cudaMalloc(&b.fine_tickets, 48 * sizeof(int)));
-    CUC(cudaMemset(b.fine_tickets, 0, 48 * sizeof(int)));
-    // the first stream carries the large chunks of device-resident input; the other two only see host-fed chunks
-    // (<= 1024 windows, pieces of a quarter of that)
-    for (int q = 0; q < 3; q++) {
-        ctx->fine_slice[q] = std::max(1, std::min(ctx->max_candidates, q == 0 ? ctx->knobs.fine_slice : std::min(ctx->knobs.fine_slice, ctx->knobs.fine_slice_side)));
-        CUC(cudaMalloc(&b.fine_state[q], (size_t)ctx->fine_slice[q] * uw_fine_state_bytes()));
-        CUC(cudaMalloc(&b.fine_pbuf[q], (size_t)ctx->fine_slice[q] * uw_fine_pbuf_bytes()));
-        CUC(cudaMalloc(&b.fine_pe[q], (size_t)ctx->fine_slice[q] * uw_fine_pe_bytes()));
-        CUC(cudaMalloc(&b.fine_pbest[q], (size_t)ctx->fine_slice[q] * uw_fine_pbest_bytes()));
-        CUC(cudaMalloc(&b.fine_tables[q], (size_t)ctx->fine_slice[q] * uw_fine_tables_bytes()));
-    }
+    // 16 384 candidates per pass on every stream: with 4 096 on the second and third, a 4 096-window host-fed chunk
+    // needed two passes (host-fed 100 000-window stream: 4 096 / 8 192 / 16 384 -> 247 / 283 / 294 k windows/s)
+    for (int q = 0; q < 3; q++) CUC(uw_fine_work_alloc(&b.fine[q], std::min(ctx->max_candidates, 16384)));
     // tables
     std::vector<float> window(UW_FFT_N);
     for (int i = 0; i < d.size; i++) window[i] = (float)sin((M_PI / (d.size - 1)) * i);  // FDR_impl.cc:103-105
@@ -765,25 +725,16 @@ int uwspr_b200_create(const uwspr_b200_params_t *params, uwspr_b200_ctx **ctx_ou
     CUC(cudaEventCreate(&ctx->ev_cp1));
     CUC(cudaEventCreate(&ctx->ev_kend));
     CUC(cudaEventCreate(&ctx->ev_end));
-    if (uw_coarse_setup(d) || uw_fine_setup() || uw_fano_setup())
+    const Knobs &kn = ctx->knobs;
+    UwFineLaunch &fl = ctx->fine_launch;
+    if (uw_coarse_setup(d) || uw_fine_setup(ctx->sm_count, !kn.no_lag_share, !kn.no_fine_reuse, &fl) || uw_fano_setup())
         return bail(fail(ctx, UWSPR_B200_E_CUDA, "cannot reserve shared memory for the kernels (not an sm_100a device?)"));
     ctx->grid_coarse = ctx->sm_count * uw_coarse_blocks_per_sm(d);
     ctx->fano_grid = ctx->sm_count * uw_fano_blocks_per_sm();
-    {
-        int bp = 1, bl = 1, bs = 1;
-        uw_fine_blocks_per_sm(&bp, &bl, &bs);
-        if (ctx->knobs.fine_ctas_per_sm > 0) {
-            bp = std::min(bp, ctx->knobs.fine_ctas_per_sm);
-            bl = std::min(bl, ctx->knobs.fine_ctas_per_sm);
-            bs = std::min(bs, ctx->knobs.fine_ctas_per_sm);
-        }
-        ctx->grid_points = ctx->sm_count * bp;
-        ctx->grid_lags = ctx->sm_count * bl;
-        ctx->grid_share = ctx->knobs.no_lag_share ? 0 : ctx->sm_count * bs;
-        if (ctx->knobs.trace)
-            fprintf(stderr, "uwspr_b200 trace: fine path: %d + %d + %d resident CTAs per SM (points, lags, lag share%s), slices of %d candidates\n",
-                    bp, bl, bs, ctx->knobs.no_lag_share ? " off" : "", std::max(1, std::min(ctx->max_candidates, ctx->knobs.fine_slice)));
-    }
+    if (kn.trace)
+        fprintf(stderr, "uwspr_b200 trace: fine path: %d + %d + %d resident CTAs per SM (points, lags, lag share%s), slices of %d candidates\n",
+                fl.grid_points / ctx->sm_count, fl.grid_lags / ctx->sm_count, fl.grid_share / ctx->sm_count,
+                fl.lag_share ? "" : " off", b.fine[0].slice);
     CUC(cudaDeviceSynchronize());
 #undef CUC
     *ctx_out = ctx;
@@ -797,11 +748,11 @@ void uwspr_b200_destroy(uwspr_b200_ctx *ctx)
     cudaSetDevice(ctx->device);
     Buffers &b = ctx->b;
     void *ptrs[] = { b.x_stage[0], b.x_stage[1], b.x_stage[2], b.amp, b.ps_dbg, b.psavg, b.peaks, b.npk, b.base, b.items,
-                     b.cands, b.refined, b.jig, b.soft, b.counters, b.fine_tickets, b.fine_state[0], b.fine_state[1], b.fine_state[2], b.fine_pbuf[0], b.fine_pbuf[1],
-                     b.fine_pbuf[2], b.fine_pe[0], b.fine_pe[1], b.fine_pe[2], b.fine_pbest[0], b.fine_pbest[1], b.fine_pbest[2], b.fine_tables[0], b.fine_tables[1], b.fine_tables[2], b.window, b.twiddle, b.off4, b.hyp_unique,
+                     b.cands, b.refined, b.jig, b.soft, b.counters, b.window, b.twiddle, b.off4, b.hyp_unique,
                      b.dec_first_ok, b.dec_tasks, b.dec_task_cycles, b.dec_task_msg, b.dec_counters, b.dec_out, b.mettab, b.rows };
     for (void *q : ptrs)
         if (q) cudaFree(q);
+    for (UwFineWork &w : b.fine) uw_fine_work_free(&w);
     for (cudaEvent_t e : ctx->ev) cudaEventDestroy(e);
     for (int q = 0; q < 3; q++) {
         if (ctx->ev_h2d[q]) cudaEventDestroy(ctx->ev_h2d[q]);

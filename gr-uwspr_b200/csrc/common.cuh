@@ -137,13 +137,28 @@ void uw_launch_worklist(const int *npk, int nwin, int cap, int *base, UwItem *it
 void uw_launch_coarse(const UwDims &d, const float *amp, const UwPeak *peaks, const UwItem *items,
                       const int *total, int cap, const uint32_t *off4, const short *hyp_unique,
                       uwspr_b200_candidate_t *cands, int *ticket, int grid, cudaStream_t s);
-// the stage sequence of the fine path over work-list entries *begin + slice0 + [0, slice_n); returns the launches issued.
-// grid_share: resident CTAs of the lag searches' shared-table kernel, 0 to run the lag searches through R1
+// The fine path's workspace for `slice` candidates (fine.cu): chain state, tone magnitudes, constant-frequency tone
+// tables and the work counters of the heavy launches.  One per compute stream: sequences on different streams run
+// concurrently.  Alloc makes one allocation and zeroes the counters; free releases it (a zeroed workspace is empty).
+struct UwFineWork {
+    void *state;                       // chain state per candidate (private to fine.cu); start of the allocation
+    float4 *pbuf, *pE, *pbest, *tables;
+    int *tickets;
+    int slice;                         // candidates one pass of the stage sequence handles
+};
+cudaError_t uw_fine_work_alloc(UwFineWork *w, int slice);
+void uw_fine_work_free(UwFineWork *w);
+// How the fine path launches, fixed when a context is created (uw_fine_setup).
+struct UwFineLaunch {
+    int grid_points, grid_lags, grid_share;   // resident CTAs of R1, R2 and R3 on the whole device
+    bool lag_share;   // the lag searches of stages A and D through R3; off: through R1 (reference path for tests)
+    bool reuse;       // stage E takes jiggle 0 from the chain; off: evaluates it again (reference path for tests)
+};
+// the stage sequence of the fine path over work-list entries *begin + slice0 + [0, w.slice); returns the launches issued
 int uw_launch_fine(const UwDims &d, const float2 *x, const UwGeom &geom, const UwItem *items, const int *begin,
                    const int *end, int cap, const uwspr_b200_candidate_t *cands, int jig_first, int jig_count,
-                   uwspr_b200_refined_t *refined, uwspr_b200_jiggle_t *jig, uint8_t *soft, int slice0, int slice_n,
-                   void *state, void *pbuf, void *pE, void *pbest, void *tables, int *tickets, int grid_points, int grid_lags,
-                   int grid_share, int reuse, cudaStream_t s);
+                   uwspr_b200_refined_t *refined, uwspr_b200_jiggle_t *jig, uint8_t *soft, int slice0,
+                   const UwFineWork &w, const UwFineLaunch &l, cudaStream_t s);
 // uwspr_b200_coarse_fine over nchan channels of device-resident samples, wins_per_chan windows each (window
 // c*wins_per_chan + k at samples + 2*(c*chan_stride + k*win_stride) floats), all jiggles' results left on the device
 // for uwspr_b200_decode_device; npk / cands are host outputs in that channel-major window order (capi.cu)
@@ -152,15 +167,10 @@ int uw_coarse_fine_channels(uwspr_b200_ctx *ctx, const float *samples, int64_t w
                             uwspr_b200_candidate_t *cands, int cap, int32_t *total);
 // kernel launches a front-end stream has issued (frontend.cu)
 int64_t uw_frontend_stream_launches(const uwspr_b200_frontend_stream *s);
-size_t uw_fine_state_bytes();  // per candidate of a slice: chain state, stage magnitudes, jiggle magnitudes
-size_t uw_fine_pbuf_bytes();
-size_t uw_fine_pe_bytes();
-size_t uw_fine_pbest_bytes();
-size_t uw_fine_tables_bytes();
-void uw_fine_blocks_per_sm(int *points, int *lags, int *share);
 size_t uw_coarse_smem_bytes(const UwDims &d);
 int uw_coarse_setup(const UwDims &d);
-int uw_fine_setup();
+// reserves the fine kernels' shared memory and fills *l for a device of sm_count SMs; nonzero on failure
+int uw_fine_setup(int sm_count, bool lag_share, bool reuse, UwFineLaunch *l);
 int uw_coarse_blocks_per_sm(const UwDims &d);
 // the Fano decoder (fano.cu).  Candidate form: task list, decoder tasks and per-candidate reduction over
 // refined[ncand], jig/soft[ncand][jig_count]; workspaces first_ok[ncand], tasks/task_cycles/task_msg

@@ -67,7 +67,7 @@ class UwsprError(RuntimeError):
 
 
 def lib_path():
-    # UWSPR_B200_LIB selects another build of the same library (kernel tuning experiments)
+    # UWSPR_B200_LIB selects another build of the same library (to compare another build with this one)
     return os.environ.get("UWSPR_B200_LIB") or os.path.join(os.path.dirname(_HERE), "libuwspr_b200.so")
 
 
