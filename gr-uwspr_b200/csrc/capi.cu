@@ -385,18 +385,20 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
     for (const UwChunk &q : chunks) use3 = use3 || q.strm == 2;
     CU(cudaEventRecord(ctx->ev_begin, cs));
     CU(cudaMemsetAsync(b.counters, 0, kCounterInts * sizeof(int), cs));
+    // caller's list: candidates before window w (the fine slices of a chunk cover exactly its own candidates)
+    std::vector<long long> first_in;
     if (!do_coarse) {
         // candidate list comes from the caller (or stays from the previous coarse call)
         if (cands_in) {
             if (!npk_in) return fail(ctx, UWSPR_B200_E_PARAM, "cands given without npk");
             if (total_in < 0) return fail(ctx, UWSPR_B200_E_PARAM, "negative candidate total");
             if (total_in > ctx->max_candidates) return fail(ctx, UWSPR_B200_E_CAPACITY, "more candidates than max_candidates");
-            long long sum = 0;
+            first_in.assign((size_t)nwin + 1, 0);
             for (int w = 0; w < nwin; w++) {
                 if (npk_in[w] < 0) return fail(ctx, UWSPR_B200_E_PARAM, "negative candidate count for a window");
-                sum += npk_in[w];
+                first_in[w + 1] = first_in[w] + npk_in[w];
             }
-            if (sum != total_in) return fail(ctx, UWSPR_B200_E_PARAM, "sum of npk differs from total");
+            if (first_in[nwin] != total_in) return fail(ctx, UWSPR_B200_E_PARAM, "sum of npk differs from total");
             CU(cudaMemcpyAsync(b.npk, npk_in, sizeof(int) * nwin, cudaMemcpyHostToDevice, cs));
             CU(cudaMemcpyAsync(b.cands, cands_in, sizeof(uwspr_b200_candidate_t) * (size_t)total_in,
                                cudaMemcpyHostToDevice, cs));
@@ -473,9 +475,12 @@ int run_impl(uwspr_b200_ctx *ctx, const float *samples, int space, int64_t win_s
         }
         CU(cudaEventRecord(e[2], st));
         if (do_fine) {
-            // the stage sequence runs over slices of at most the workspace's slice of candidates; the number of
-            // candidates is a device value, so the launches cover the most the chunk can hold
-            const long long most = std::min<long long>(ctx->max_candidates, (long long)nw * d.maxcand);
+            // the stage sequence runs over slices of at most the workspace's slice of candidates.  A list from the
+            // coarse search has at most maxcand candidates per window, but its length is a device value, so the
+            // launches cover the most the chunk can hold; the caller's list may give a window any number of
+            // candidates (the reference takes them all), and its chunk counts are known here
+            const long long held = first_in.empty() ? (long long)nw * d.maxcand : first_in[w0 + nw] - first_in[w0];
+            const long long most = std::min<long long>(ctx->max_candidates, held);
             const UwFineWork &fw = b.fine[ch.strm];
             for (long long s0 = 0; s0 < most; s0 += fw.slice)
                 ctx->launches += uw_launch_fine(d, xfine, geom, b.items, set + 1, set + 2, ctx->max_candidates, b.cands,
