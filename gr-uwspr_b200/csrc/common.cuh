@@ -165,6 +165,26 @@ int uw_launch_fine(const UwDims &d, const float2 *x, const UwGeom &geom, const U
 int uw_coarse_fine_channels(uwspr_b200_ctx *ctx, const float *samples, int64_t win_stride, int wins_per_chan,
                             int64_t chan_stride, int nchan, int jig_first, int jig_count, int32_t *npk,
                             uwspr_b200_candidate_t *cands, int cap, int32_t *total);
+// A delay-and-sum beam set on the device (beam.cu): weights and delays regrouped for k_beamform.
+#define UW_BEAM_MAX_DELAY 8192
+struct UwBeams {
+    float2 *w = nullptr;
+    int *d = nullptr;
+    int2 *span = nullptr;          // per (beam group, channel): smallest and largest delay
+    int nbeam = 0, nchan = 0, ngroup = 0;
+    int maxspan = 0, dmax = 0;     // widest delay range of a group on one channel; largest delay
+    size_t smem = 0;               // dynamic shared memory of a launch
+};
+// E_PARAM unless 1 <= nchan, nbeam <= 1024, the pointers are set, every weight is finite and every delay in
+// [0, UW_BEAM_MAX_DELAY]; no CUDA call
+int uw_beams_check(int nchan, const float *weights, const int32_t *delays, int nbeam);
+// weights: nbeam*nchan (re, im) pairs, beam-major; delays: nbeam*nchan.  Host pointers, arguments already checked.
+cudaError_t uw_beams_upload(UwBeams *b, int nchan, const float *weights, const int32_t *delays, int nbeam);
+void uw_beams_free(UwBeams *b);
+// beam b's outputs j in [0, n_out) to out + b*out_stride + j: y_b[j] = sum_c w[b][c] x_c, x_c read at
+// in + c*in_stride + h + j - d[b][c], zero where that index is negative
+void uw_launch_beamform(const UwBeams &b, const float2 *in, long long in_stride, long long h, float2 *out,
+                        long long out_stride, long long n_out, cudaStream_t s);
 // kernel launches a front-end stream has issued (frontend.cu)
 int64_t uw_frontend_stream_launches(const uwspr_b200_frontend_stream *s);
 size_t uw_coarse_smem_bytes(const UwDims &d);

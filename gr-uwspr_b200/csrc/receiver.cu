@@ -8,6 +8,13 @@
 // then the decoder on the results left on the device.  The unread tail of every row then moves to the front of
 // the second buffer, which becomes the ring: source and destination would overlap within one buffer whenever
 // the tail is longer than K*stride (41 625 samples at shift 9 s and K = 1).
+//
+// Beams (uwspr_b200_array_receiver_create_beams): the ring's rows are nbeam delay-and-sum beams of the nchan channels.
+// The channels' new samples go to a staging area instead, [nchan][spitch], whose rows hold the last nhist <= dmax
+// samples of each channel (dmax = the largest delay) followed by the push piece.  One k_beamform launch per piece reads
+// x_c[n - d] from there (beam.cu: output n depends on n and the inputs alone, so the beams equal uwspr_b200_beamform
+// over the whole input whatever the split) and appends the piece's beam samples to the ring.  The last dmax samples
+// of every staged row then move to the front of the second staging buffer, as the ring's tail does.
 #include <string.h>
 
 #include <algorithm>
@@ -22,7 +29,9 @@ namespace {
 // when a push piece starts, since every complete batch has been run by then
 constexpr int64_t kRingPiece = 16384;
 
-int check_args(const uwspr_b200_params_t *p, const uwspr_b200_input_t *in, int nchan, int shift_seconds, int batch_windows)
+// nrow: rows of the ring (nchan, or nbeam with beams)
+int check_args(const uwspr_b200_params_t *p, const uwspr_b200_input_t *in, int nchan, int nrow, int shift_seconds,
+               int batch_windows)
 {
     if (!p || !in || nchan < 1 || batch_windows < 1 || p->fs <= 0) return UWSPR_B200_E_PARAM;
     const long long stride = (long long)shift_seconds * p->fs;
@@ -33,8 +42,16 @@ int check_args(const uwspr_b200_params_t *p, const uwspr_b200_input_t *in, int n
             !(in->fs_in > 0.0) || in->fs_in / in->decim != (double)p->fs)
             return UWSPR_B200_E_PARAM;
     }
-    if ((long long)nchan * batch_windows > INT_MAX / 2) return UWSPR_B200_E_PARAM;
+    if ((long long)nrow * batch_windows > INT_MAX / 2) return UWSPR_B200_E_PARAM;
     return UWSPR_B200_OK;
+}
+
+int check_all(const uwspr_b200_params_t *p, const uwspr_b200_input_t *in, int nchan, const uwspr_b200_beams_t *beams,
+              int shift_seconds, int batch_windows)
+{
+    if (!beams) return check_args(p, in, nchan, nchan, shift_seconds, batch_windows);
+    const int st = uw_beams_check(nchan, beams->weights, beams->delays, beams->nbeam);
+    return st ? st : check_args(p, in, nchan, beams->nbeam, shift_seconds, batch_windows);
 }
 
 void cuda_check(cudaError_t e, const char *what)
@@ -48,18 +65,19 @@ namespace gr {
 namespace uwspr {
 
 array_receiver::array_receiver(const uwspr_b200_params_t &params, const uwspr_b200_input_t &input, int nchan, int shift_seconds,
-                               int batch_windows)
+                               int batch_windows, const uwspr_b200_beams_t *beams)
 {
-    int st = check_args(&params, &input, nchan, shift_seconds, batch_windows);
+    int st = check_all(&params, &input, nchan, beams, shift_seconds, batch_windows);
     if (st) throw context_error(st, "bad receiver arguments");
     d_device = params.device;
     d_kind = input.kind;
     d_nchan = nchan;
+    d_nrow = beams ? beams->nbeam : nchan;
     d_fl = params.fl;
     d_stride = shift_seconds * params.fs;
     d_batch = batch_windows;
     uwspr_b200_params_t p = params;
-    p.max_windows = nchan * batch_windows;
+    p.max_windows = d_nrow * batch_windows;
     try {
         st = uwspr_b200_create(&p, &d_ctx);
         if (st) throw context_error(st, uwspr_b200_create_error());
@@ -75,7 +93,15 @@ array_receiver::array_receiver(const uwspr_b200_params_t &params, const uwspr_b2
         // rows start on 64-sample boundaries: every channel's windows keep the alignment a single stream's have
         d_pitch = ((int64_t)(batch_windows - 1) * d_stride + d_fl + kRingPiece + 63) / 64 * 64;
         cuda_check(cudaSetDevice(params.device), "cudaSetDevice");
-        for (int q = 0; q < 2; q++) cuda_check(cudaMalloc(&d_ring[q], (size_t)nchan * d_pitch * sizeof(float2)), "cudaMalloc");
+        for (int q = 0; q < 2; q++) cuda_check(cudaMalloc(&d_ring[q], (size_t)d_nrow * d_pitch * sizeof(float2)), "cudaMalloc");
+        if (beams) {
+            d_beamed = true;
+            d_beams = new UwBeams();
+            cuda_check(uw_beams_upload(d_beams, nchan, beams->weights, beams->delays, beams->nbeam), "beam tables");
+            d_spitch = (d_beams->dmax + kRingPiece + 63) / 64 * 64;
+            for (int q = 0; q < 2; q++)
+                cuda_check(cudaMalloc(&d_stage[q], (size_t)nchan * d_spitch * sizeof(float2)), "cudaMalloc");
+        }
         cudaStream_t s;
         cuda_check(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking), "cudaStreamCreate");
         d_stream = s;
@@ -83,7 +109,7 @@ array_receiver::array_receiver(const uwspr_b200_params_t &params, const uwspr_b2
         release();
         throw;
     }
-    d_npk.resize((size_t)nchan * batch_windows);
+    d_npk.resize((size_t)d_nrow * batch_windows);
     d_cands.resize(d_cap);
     d_decoded.resize(d_cap);
     d_blobs.resize((size_t)d_cap * 7);
@@ -102,13 +128,25 @@ void array_receiver::release()
         if (q) cudaFree(q);
         q = nullptr;
     }
+    for (void *&q : d_stage) {
+        if (q) cudaFree(q);
+        q = nullptr;
+    }
+    if (d_beams) {
+        uw_beams_free(d_beams);
+        delete d_beams;
+        d_beams = nullptr;
+    }
     uwspr_b200_frontend_stream_destroy(d_fe);
     d_fe = nullptr;
     uwspr_b200_destroy(d_ctx);
     d_ctx = nullptr;
 }
 
-int64_t array_receiver::launch_count() const { return uwspr_b200_launch_count(d_ctx) + uw_frontend_stream_launches(d_fe); }
+int64_t array_receiver::launch_count() const
+{
+    return uwspr_b200_launch_count(d_ctx) + uw_frontend_stream_launches(d_fe) + d_beam_launches;
+}
 
 void array_receiver::push(const void *data, int space, int64_t chan_stride, int64_t n)
 {
@@ -116,14 +154,16 @@ void array_receiver::push(const void *data, int space, int64_t chan_stride, int6
     cuda_check(cudaSetDevice(d_device), "cudaSetDevice");
     const size_t esz = d_kind == 0 ? sizeof(float2) : d_kind == 1 ? sizeof(float) : sizeof(short);
     for (int64_t off = 0; off < n;) {
-        // the ring has room for kRingPiece samples at least (process() ran every complete batch)
-        float2 *row0 = static_cast<float2 *>(d_ring[d_cur]) + d_fill;
-        const int64_t room = d_pitch - d_fill;
+        // the ring has room for kRingPiece samples at least (process() ran every complete batch); with beams the
+        // channels' samples go to the staging rows, after their history, and a piece is at most kRingPiece samples
+        float2 *row0 = d_beamed ? static_cast<float2 *>(d_stage[d_scur]) + d_nhist : static_cast<float2 *>(d_ring[d_cur]) + d_fill;
+        const int64_t pitch = d_beamed ? d_spitch : d_pitch;
+        const int64_t room = d_beamed ? std::min(kRingPiece, d_pitch - d_fill) : d_pitch - d_fill;
         const char *src = static_cast<const char *>(data) + (size_t)off * esz;
         int64_t take, got;
         if (d_kind == 0) {
             take = got = std::min(room, n - off);
-            cuda_check(cudaMemcpy2DAsync(row0, (size_t)d_pitch * sizeof(float2), src, (size_t)chan_stride * esz,
+            cuda_check(cudaMemcpy2DAsync(row0, (size_t)pitch * sizeof(float2), src, (size_t)chan_stride * esz,
                                          (size_t)take * sizeof(float2), (size_t)d_nchan,
                                          space == UWSPR_B200_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, st),
                        "cudaMemcpy2DAsync");
@@ -132,13 +172,35 @@ void array_receiver::push(const void *data, int space, int64_t chan_stride, int6
             // take samples produce at most ceil(take / decim) <= room outputs
             take = std::min(n - off, room * d_decim);
             const int rc = uwspr_b200_frontend_stream_push(d_fe, src, space, chan_stride, take, reinterpret_cast<float *>(row0),
-                                                           UWSPR_B200_DEVICE, d_pitch, room, &got);
+                                                           UWSPR_B200_DEVICE, pitch, room, &got);
             if (rc) throw context_error(rc, uwspr_b200_frontend_error());
         }
         off += take;
+        if (d_beamed) beamform_piece(got);
         d_fill += got;
         process(false);
     }
+}
+
+// the piece's `got` new samples of every channel are in the staging rows after d_nhist samples of history
+void array_receiver::beamform_piece(int64_t got)
+{
+    if (got == 0) return;
+    cudaStream_t st = static_cast<cudaStream_t>(d_stream);
+    const float2 *stage = static_cast<const float2 *>(d_stage[d_scur]);
+    uw_launch_beamform(*d_beams, stage, d_spitch, d_nhist, static_cast<float2 *>(d_ring[d_cur]) + d_fill, d_pitch, got, st);
+    d_beam_launches++;
+    cuda_check(cudaGetLastError(), "k_beamform");
+    // the next piece reads back at most dmax samples: keep the last of (history, piece), in the other buffer
+    const int64_t keep = std::min<int64_t>(d_beams->dmax, d_nhist + got);
+    if (keep > 0)
+        cuda_check(cudaMemcpy2DAsync(d_stage[d_scur ^ 1], (size_t)d_spitch * sizeof(float2), stage + (d_nhist + got - keep),
+                                     (size_t)d_spitch * sizeof(float2), (size_t)keep * sizeof(float2), (size_t)d_nchan,
+                                     cudaMemcpyDeviceToDevice, st),
+                   "cudaMemcpy2DAsync");
+    cuda_check(cudaStreamSynchronize(st), "cudaStreamSynchronize");
+    d_scur ^= 1;
+    d_nhist = keep;
 }
 
 void array_receiver::flush() { process(true); }
@@ -156,17 +218,17 @@ void array_receiver::run_batch(int nb)
 {
     const float *ring = static_cast<const float *>(d_ring[d_cur]);
     int32_t total = 0;
-    int st = uw_coarse_fine_channels(d_ctx, ring, d_stride, nb, d_pitch, d_nchan, 0, UWSPR_B200_NJIG, d_npk.data(),
+    int st = uw_coarse_fine_channels(d_ctx, ring, d_stride, nb, d_pitch, d_nrow, 0, UWSPR_B200_NJIG, d_npk.data(),
                                      d_cands.data(), d_cap, &total);
     if (st) throw context_error(st, uwspr_b200_last_error(d_ctx));
     const int got = uwspr_b200_decode_device(d_ctx, nullptr, nullptr, nullptr, UWSPR_B200_DEVICE, total, UWSPR_B200_NJIG,
                                              d_decoded.data(), d_blobs.data(), nullptr, nullptr);
     if (got < 0) throw context_error(-got, uwspr_b200_last_error(d_ctx));
-    // results are channel-major (window c*nb + k); messages are published window by window, channel by channel
-    std::vector<int> base((size_t)d_nchan * nb + 1, 0);
-    for (int i = 0; i < d_nchan * nb; i++) base[i + 1] = base[i] + d_npk[i];
+    // results are row-major (window c*nb + k); messages are published window by window, row by row
+    std::vector<int> base((size_t)d_nrow * nb + 1, 0);
+    for (int i = 0; i < d_nrow * nb; i++) base[i + 1] = base[i] + d_npk[i];
     for (int k = 0; k < nb; k++)
-        for (int c = 0; c < d_nchan; c++)
+        for (int c = 0; c < d_nrow; c++)
             for (int g = base[c * nb + k]; g < base[c * nb + k + 1]; g++) {
                 if (!d_decoded[g]) continue;
                 message_pdu m;
@@ -181,7 +243,7 @@ void array_receiver::run_batch(int nb)
     cudaStream_t s = static_cast<cudaStream_t>(d_stream);
     if (tail > 0) {
         cuda_check(cudaMemcpy2DAsync(d_ring[d_cur ^ 1], (size_t)d_pitch * sizeof(float2), ring + 2 * done,
-                                     (size_t)d_pitch * sizeof(float2), (size_t)tail * sizeof(float2), (size_t)d_nchan,
+                                     (size_t)d_pitch * sizeof(float2), (size_t)tail * sizeof(float2), (size_t)d_nrow,
                                      cudaMemcpyDeviceToDevice, s),
                    "cudaMemcpy2DAsync");
         cuda_check(cudaStreamSynchronize(s), "cudaStreamSynchronize");
@@ -226,13 +288,13 @@ template <class F> int guarded(F &&f)
 }
 
 int create(const uwspr_b200_params_t *params, const uwspr_b200_input_t *input, int nchan, int shift_seconds, int batch_windows,
-           rx_handle **out)
+           rx_handle **out, const uwspr_b200_beams_t *beams = nullptr)
 {
     if (!out) return UWSPR_B200_E_PARAM;
     *out = nullptr;
-    const int st = check_args(params, input, nchan, shift_seconds, batch_windows);
+    const int st = check_all(params, input, nchan, beams, shift_seconds, batch_windows);
     if (st) return st;
-    return guarded([&] { *out = new rx_handle(*params, *input, nchan, shift_seconds, batch_windows); });
+    return guarded([&] { *out = new rx_handle(*params, *input, nchan, shift_seconds, batch_windows, beams); });
 }
 
 int push(rx_handle *h, const void *data, int space, int64_t chan_stride, int64_t n, int flush)
@@ -255,6 +317,17 @@ int uwspr_b200_array_receiver_create(const uwspr_b200_params_t *params, const uw
                                      int shift_seconds, int batch_windows, uwspr_b200_array_receiver **out)
 {
     return create(params, input, nchan, shift_seconds, batch_windows, reinterpret_cast<rx_handle **>(out));
+}
+
+int uwspr_b200_array_receiver_create_beams(const uwspr_b200_params_t *params, const uwspr_b200_input_t *input, int nchan,
+                                           const uwspr_b200_beams_t *beams, int shift_seconds, int batch_windows,
+                                           uwspr_b200_array_receiver **out)
+{
+    if (!beams) {
+        if (out) *out = nullptr;
+        return UWSPR_B200_E_PARAM;
+    }
+    return create(params, input, nchan, shift_seconds, batch_windows, reinterpret_cast<rx_handle **>(out), beams);
 }
 
 void uwspr_b200_array_receiver_destroy(uwspr_b200_array_receiver *rx) { delete reinterpret_cast<rx_handle *>(rx); }

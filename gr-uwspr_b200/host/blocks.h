@@ -32,6 +32,8 @@
 
 #include "uwspr_b200.h"
 
+struct UwBeams;
+
 namespace gr {
 namespace uwspr {
 
@@ -123,12 +125,14 @@ private:
 
 // Receive chain of nchan channels in lockstep: front-end stream -> ring of 375-sps streams on the device ->
 // one coarse+fine submission per `batch` windows of every channel -> decoder on the device.
+// With beams, the channels go to a staging area and the ring holds nbeam delay-and-sum beams of them instead: the rest
+// of the chain sees one 375-sps stream per beam.
 class array_receiver
 {
 public:
-    // throws context_error (E_PARAM for the checks of uwspr_b200_array_receiver_create)
+    // throws context_error (E_PARAM for the checks of uwspr_b200_array_receiver_create[_beams]); beams may be NULL
     array_receiver(const uwspr_b200_params_t &params, const uwspr_b200_input_t &input, int nchan, int shift_seconds,
-                   int batch_windows);
+                   int batch_windows, const uwspr_b200_beams_t *beams = nullptr);
     ~array_receiver();
     // n samples of every channel, channel c at data + c*chan_stride samples; runs a submission whenever `batch`
     // complete windows are buffered on every channel
@@ -143,12 +147,21 @@ private:
     void release();
     void process(bool all);
     void run_batch(int per_chan);
+    void beamform_piece(int64_t got);
     uwspr_b200_ctx *d_ctx = nullptr;
     uwspr_b200_frontend_stream *d_fe = nullptr;
     void *d_stream = nullptr;                // cudaStream_t of the ring copies
-    void *d_ring[2] = { nullptr, nullptr };  // complex64 [nchan][d_pitch]: the ring and the buffer its tail moves to
+    void *d_ring[2] = { nullptr, nullptr };  // complex64 [nrow][d_pitch]: the ring and the buffer its tail moves to
     int d_cur = 0;
     int d_device, d_kind, d_nchan, d_fl, d_stride, d_batch, d_cap, d_decim = 1;
+    int d_nrow;                              // rows of the ring: nbeam with beams, else nchan
+    // beams: the channels' streams go to d_stage (complex64 [nchan][d_spitch]), whose rows hold the last d_nhist
+    // samples (at most the largest delay) followed by the current push piece; the history moves to the other buffer
+    bool d_beamed = false;
+    UwBeams *d_beams = nullptr;
+    void *d_stage[2] = { nullptr, nullptr };
+    int d_scur = 0;
+    int64_t d_spitch = 0, d_nhist = 0, d_beam_launches = 0;
     int64_t d_pitch = 0, d_fill = 0;         // samples per channel of the ring, and those held (from window d_next_window)
     int64_t d_next_window = 0;
     std::deque<message_pdu> d_msgs;

@@ -24,7 +24,7 @@ EXPORTED_SYMBOLS = [
     "uwspr_b200_frontend_stream_create", "uwspr_b200_frontend_stream_push", "uwspr_b200_frontend_stream_outputs",
     "uwspr_b200_frontend_stream_destroy", "uwspr_b200_array_receiver_create", "uwspr_b200_array_receiver_push",
     "uwspr_b200_array_receiver_pop", "uwspr_b200_array_receiver_windows", "uwspr_b200_array_receiver_launch_count",
-    "uwspr_b200_array_receiver_destroy",
+    "uwspr_b200_array_receiver_destroy", "uwspr_b200_beamform", "uwspr_b200_array_receiver_create_beams",
 ]
 
 CAND_DTYPE = np.dtype(
@@ -49,6 +49,10 @@ class Params(C.Structure):
 class Input(C.Structure):
     _fields_ = [("kind", C.c_int32), ("taps", C.c_void_p), ("ntaps", C.c_int32), ("complex_taps", C.c_int32),
                 ("decim", C.c_int32), ("delay", C.c_int32), ("fc", C.c_double), ("fs_in", C.c_double)]
+
+
+class Beams(C.Structure):
+    _fields_ = [("nbeam", C.c_int32), ("weights", C.c_void_p), ("delays", C.c_void_p)]
 
 
 class Info(C.Structure):
@@ -171,6 +175,11 @@ def load_library():
     L.uwspr_b200_array_receiver_launch_count.restype = i64
     L.uwspr_b200_array_receiver_launch_count.argtypes = [vp]
     L.uwspr_b200_array_receiver_destroy.argtypes = [vp]
+    L.uwspr_b200_array_receiver_create_beams.restype = C.c_int
+    L.uwspr_b200_array_receiver_create_beams.argtypes = [C.POINTER(Params), C.POINTER(Input), C.c_int, C.POINTER(Beams), C.c_int,
+                                                         C.c_int, C.POINTER(vp)]
+    L.uwspr_b200_beamform.restype = C.c_int
+    L.uwspr_b200_beamform.argtypes = [C.c_int, vp, C.c_int, i64, C.c_int, i64, vp, vp, C.c_int, vp, C.c_int, i64]
     L.uwspr_b200_hashtab_bytes.restype = C.c_size_t
     L.uwspr_b200_unpack.restype = C.c_int
     L.uwspr_b200_unpack.argtypes = [vp, vp, vp, C.c_size_t]
@@ -737,15 +746,70 @@ class FrontendStream:
 _INPUT_KINDS = {"complex64": (0, np.complex64), "float32": (1, np.float32), "int16": (2, np.int16)}
 
 
+def _beam_tables(weights, delays, nchan=None):
+    """(weights as [nbeam, nchan] complex64, delays as [nbeam, nchan] int32); the shapes must agree"""
+    w = np.ascontiguousarray(weights, dtype=np.complex64)
+    d = np.ascontiguousarray(delays, dtype=np.int32)
+    if w.ndim != 2 or d.shape != w.shape or (nchan is not None and w.shape[1] != nchan):
+        raise ValueError("weights and delays must both be [nbeam, nchan]%s" % ("" if nchan is None else " with nchan %d" % nchan))
+    return w, d
+
+
+def beamform(x, weights, delays, device=0, out_device_ptr=None, out_stride=None):
+    """delay-and-sum beams on the GPU (uwspr_b200_beamform): y_b[n] = sum_c weights[b, c] x_c[n - delays[b, c]], x_c = 0
+    before its first sample.  x: numpy [nchan, n] complex64, or a (device pointer, dtype, shape) tuple as frontend()
+    accepts; weights [nbeam, nchan] complex, delays [nbeam, nchan] integers in [0, 8192].  Returns complex64
+    [nbeam, n], or n when out_device_ptr is given (beam b is then written at out_device_ptr + 8*b*out_stride bytes)."""
+    L = load_library()
+    ptr, space, keep, nchan, n, stride = _channels_arg(x, np.complex64)
+    w, d = _beam_tables(weights, delays, nchan)
+    nbeam = w.shape[0]
+    if out_device_ptr is None:
+        out = np.zeros((nbeam, n), np.complex64)
+        optr, ospace, ostride = _p(out), HOST, n
+    else:
+        out, optr, ospace = None, C.c_void_p(int(out_device_ptr)), DEVICE
+        ostride = n if out_stride is None else int(out_stride)
+    st = L.uwspr_b200_beamform(device, ptr, space, stride, nchan, n, _p(w), _p(d), nbeam, optr, ospace, ostride)
+    if st != 0:
+        raise UwsprError(st, L.uwspr_b200_status_string(st).decode())
+    return n if out is None else out
+
+
+def plane_wave_steering(positions_m, directions, sound_speed=1500.0, fc=1500.0, fs=375.0):
+    """(weights [nbeam, nchan] complex64, delays [nbeam, nchan] int32) of delay-and-sum beams steered at plane waves.
+    positions_m: [nchan, 2 or 3] hydrophone positions in metres; directions: [nbeam, same dimension] unit vectors
+    pointing from the array towards each source.  A plane wave from u reaches hydrophone c at tau_c = -(p_c . u) / c_s
+    (relative to the origin).  Beam b delays channel c by d_c = round((tau_max - tau_c) fs) samples at baseband, so
+    that every channel lines up with the last arrival, and its weight removes the carrier phase of the whole
+    alignment delay tau_max - tau_c, integer part and residual fraction: after the mix-down by fc a passband delay tau
+    is the phase e^{-i 2 pi fc tau} (the envelope error left by rounding is under half a sample).  Weights are
+    normalised to sum |w_c|^2 = 1, so a beam's noise level in independent noise equals one hydrophone's."""
+    p = np.asarray(positions_m, dtype=np.float64)
+    u = np.asarray(directions, dtype=np.float64)
+    if u.ndim == 1:
+        u = u[None, :]
+    if p.ndim != 2 or u.ndim != 2 or p.shape[1] != u.shape[1] or p.shape[1] not in (2, 3):
+        raise ValueError("positions [nchan, 2 or 3] and directions [nbeam, same dimension]")
+    tau = -(u @ p.T) / sound_speed                       # [nbeam, nchan] arrival times, s
+    align = tau.max(axis=1, keepdims=True) - tau         # delay that lines channel c up with the last arrival
+    delays = np.rint(align * fs).astype(np.int32)
+    weights = np.exp(-2j * np.pi * fc * align) / np.sqrt(p.shape[0])
+    return weights.astype(np.complex64), delays
+
+
 class ArrayReceiver:
     """receive chain of nchan channels in lockstep (uwspr_b200_array_receiver): 375-sps complex64 input, or float32 /
     int16 audio at fs_in through the front-end stream (taps, decim, fc, delay as for frontend()); sliding windows of
     `shift` seconds, batch_windows windows of every channel per submission, decoded on the device.
-    push(data [nchan, n], flush) returns [(channel, window, message7, candidate)] in (window, channel, candidate) order."""
+    push(data [nchan, n], flush) returns [(channel, window, message7, candidate)] in (window, channel, candidate) order.
+    beams=(weights [nbeam, nchan] complex64, delays [nbeam, nchan] int32) decodes nbeam delay-and-sum beams of the
+    channels instead (uwspr_b200_array_receiver_create_beams; plane_wave_steering makes them): `channel` is then the
+    beam index, and the order is (window, beam, candidate)."""
 
     def __init__(self, nchan, fs=375, fl=45000, spb=256, maxdrift=0, maxfreqs=200, halfbandwidth=10, cf=1500, threshold=10,
                  shift=9, batch_windows=16, input="complex64", taps=None, decim=32, fc=1500.0, fs_in=12000.0, delay=None,
-                 device=0, max_candidates=0):
+                 device=0, max_candidates=0, beams=None):
         self.L = load_library()
         kind, self.dtype = _INPUT_KINDS[input]
         prm = Params(fs, fl, spb, maxdrift, maxfreqs, halfbandwidth, cf, threshold, device, 0, max_candidates, 0)
@@ -756,7 +820,13 @@ class ArrayReceiver:
             inp = Input(kind, _p(self.taps), len(self.taps), int(ctaps), decim, delay, fc, fs_in)
         self.nchan = nchan
         h = C.c_void_p()
-        st = self.L.uwspr_b200_array_receiver_create(C.byref(prm), C.byref(inp), nchan, shift, batch_windows, C.byref(h))
+        if beams is None:
+            st = self.L.uwspr_b200_array_receiver_create(C.byref(prm), C.byref(inp), nchan, shift, batch_windows, C.byref(h))
+        else:
+            w, d = _beam_tables(*beams, nchan=nchan)
+            bm = Beams(w.shape[0], _p(w), _p(d))
+            st = self.L.uwspr_b200_array_receiver_create_beams(C.byref(prm), C.byref(inp), nchan, C.byref(bm), shift,
+                                                                batch_windows, C.byref(h))
         if st != 0:
             text = self.L.uwspr_b200_create_error().decode() if st == 2 else ""
             raise UwsprError(st, text or self.L.uwspr_b200_status_string(st).decode())

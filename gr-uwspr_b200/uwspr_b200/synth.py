@@ -127,3 +127,41 @@ def gen_array(chan_lo, chan_hi, nwin, whales, device, stream_id=64, snr_db=-21.0
             x[p0:p0 + m] += gain * sig[:m]
             out[c - chan_lo, w] = x
     return out, truth
+
+
+def gen_plane_wave_audio(positions_m, direction, nchan, minutes, snr_db_per_channel, seed, message=("K1ABC", "FN42", 37),
+                         f0=2.0, start_s=1.0, fs_in=12000.0, fc=1500.0, sound_speed=1500.0, noise_rms=0.2, fmt="int16"):
+    """Audio of a hydrophone array hearing one WSPR transmitter as a plane wave, in independent noise per hydrophone.
+    positions_m [nchan, 2 or 3] in metres; direction: unit vector from the array towards the source.  Hydrophone c hears
+    the source at tau_c = -(p_c . u) / sound_speed (relative to the origin): its audio is cos(2 pi int_0^{t - tau_c} f),
+    evaluated in float64 from the exact fractional delay (no integer shift at baseband), with f = fc + f0 +
+    (symbol - 1.5) * 375/256 Hz for the 162 symbols of `message` from start_s on.  Each channel adds Gaussian noise of
+    rms noise_rms (full scale 1) from its own generator, default_rng([seed, c]); snr_db_per_channel is the signal's
+    power over the noise power in 2500 Hz, as WSPR states SNR.  fmt "int16" (PCM, x 32768, clipped) or "float32".
+    Returns (audio [nchan, n], dict(msg=7 bytes, text, tau=[nchan] seconds, amplitude))."""
+    from .binding import channel_symbols, pack_type1
+    p = np.asarray(positions_m, dtype=np.float64)
+    u = np.asarray(direction, dtype=np.float64)
+    if p.shape != (nchan, u.size) or u.size not in (2, 3):
+        raise ValueError("positions_m must be [nchan, 2 or 3] and direction of the same dimension")
+    n = int(minutes * 60 * fs_in)
+    tau = -(p @ u) / sound_speed
+    msg = pack_type1(*message)
+    sym = channel_symbols(msg).astype(np.float64)
+    tsym = SPS / FS
+    f = fc + f0 + (sym - 1.5) * FS / SPS                          # Hz, per symbol
+    cyc0 = np.concatenate([[0.0], np.cumsum(f * tsym)])            # cycles at the start of each symbol
+    amp = np.sqrt(2.0 * 10 ** (snr_db_per_channel / 10.0) * noise_rms ** 2 * 2500.0 / (fs_in / 2.0))
+    t = np.arange(n, dtype=np.float64) / fs_in
+    out = np.empty((nchan, n), np.int16 if fmt == "int16" else np.float32)
+    for c in range(nchan):
+        tp = t - tau[c] - start_s                                  # time since the first symbol, at this hydrophone
+        k = np.floor(tp / tsym)
+        on = (k >= 0) & (k < NSYM)
+        ki = np.where(on, k, 0).astype(np.int64)
+        cyc = cyc0[ki] + f[ki] * (tp - ki * tsym)
+        a = np.where(on, amp * np.cos(2 * np.pi * (cyc - np.floor(cyc))), 0.0)
+        a += np.random.default_rng([seed, c]).normal(0.0, noise_rms, n)
+        out[c] = np.clip(np.round(a * 32768.0), -32768, 32767) if fmt == "int16" else a
+    text = "%s %s %2d" % message
+    return out, dict(msg=bytes(msg), text=text, tau=tau, amplitude=amp)

@@ -363,6 +363,42 @@ UWSPR_B200_API int64_t uwspr_b200_array_receiver_windows(const uwspr_b200_array_
 UWSPR_B200_API int64_t uwspr_b200_array_receiver_launch_count(const uwspr_b200_array_receiver *rx);
 UWSPR_B200_API void uwspr_b200_array_receiver_destroy(uwspr_b200_array_receiver *rx);
 
+/* ---- delay-and-sum beams of a hydrophone array ------------------------------------------------------------------
+ * Narrowband delay-and-sum at complex baseband, nbeam beams from nchan channels:
+ *     y_b[n] = sum_{c=0}^{nchan-1} w[b][c] * x_c[n - d[b][c]],   x_c[m] = 0 for m < 0,
+ * w complex, d an integer sample delay.  After the front-end's mix-down by fc, a passband delay tau is a delay of the
+ * envelope and the phase e^{-i 2 pi fc tau}, so integer delays and complex weights steer any geometry to within half a
+ * sample of envelope error (uwspr_b200.plane_wave_steering computes them for a plane wave).  Each output is an fmaf
+ * chain over ascending c that starts at (0, 0): re += wr*xr, re += -wi*xi, im += wr*xi, im += wi*xr, one rounding each.
+ * So an output does not depend on how the work is split, and a stream of beams (the receiver below) equals this
+ * one-shot form bit for bit.
+ * in: complex64, channel c at in + 2*c*in_stride floats, n samples each, in `space_in`; out: complex64, beam b at
+ * out + 2*b*out_stride floats, in `space_out` (a device output feeds uwspr_b200_coarse_fine directly).  weights
+ * (nbeam*nchan (re, im) pairs, beam-major) and delays (nbeam*nchan) are host pointers.
+ * E_PARAM before any CUDA call: nchan or nbeam outside 1..1024, a weight that is not finite, a delay outside
+ * [0, 8192], a NULL pointer, n < 0, in_stride < n, out_stride < n or a bad space. */
+UWSPR_B200_API int uwspr_b200_beamform(int device, const float *in, int space_in, int64_t in_stride, int nchan, int64_t n,
+                                       const float *weights, const int32_t *delays, int nbeam, float *out, int space_out,
+                                       int64_t out_stride);
+/* A beam set for the receiver: weights and delays as for uwspr_b200_beamform (host pointers, copied at create). */
+typedef struct {
+    int32_t nbeam;
+    const float *weights;    /* nbeam*nchan (re, im) pairs, beam-major */
+    const int32_t *delays;   /* nbeam*nchan samples in [0, 8192] */
+} uwspr_b200_beams_t;
+/* The array receiver on beams instead of channels.  The channels' streams (any input kind) go to a staging area on
+ * the device that keeps the last max(delays) samples of each; after every push piece one beamformer launch appends
+ * the new samples of every beam y_b to the ring, which holds nbeam rows.  Window k of beam b is
+ * y_b[k*shift*fs, k*shift*fs + fl), and everything downstream is the array receiver's: pop returns the beam index in
+ * `channel`, messages come out in (window, beam, candidate) order without de-duplication and do not depend on
+ * batch_windows or on how the input is split into pushes.  params->max_windows is ignored (nbeam * batch_windows).
+ * push, pop, windows, launch_count (beamformer launches included) and destroy are the functions above.
+ * E_PARAM before any CUDA call: the checks of uwspr_b200_array_receiver_create, a NULL beams, those of
+ * uwspr_b200_beamform on nchan, nbeam, weights and delays, and nbeam * batch_windows > INT_MAX / 2. */
+UWSPR_B200_API int uwspr_b200_array_receiver_create_beams(const uwspr_b200_params_t *params, const uwspr_b200_input_t *input,
+                                                          int nchan, const uwspr_b200_beams_t *beams, int shift_seconds,
+                                                          int batch_windows, uwspr_b200_array_receiver **out);
+
 /* ---- utilities ------------------------------------------------------------------------- */
 /* pinned host memory for sample / result buffers (cudaHostAlloc / cudaFreeHost) */
 UWSPR_B200_API int uwspr_b200_host_alloc(void **ptr, size_t bytes);
